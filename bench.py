@@ -10,7 +10,7 @@ One *eval* = one (J_k, grad J_k) pair of ONE component over all N samples, i.e. 
 the ensemble).  With --gpus N the 64 components are sharded over the ranks (strong scaling, no
 data-path collective); value = 64 * steps / max-over-ranks device time.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 `--impl reference` times the CPU port of the reference algorithm (oracle/ttm_oracle.py, component-
 parallel over all host cores like the reference's multiprocessing Pool, tm.py:2789-2845) on a bounded
@@ -518,6 +518,30 @@ def extras(torch, with_cpu=True):
     return out
 
 
+def step_outputs(tm, ks, coefs, world, dist, torch):
+    """What the last launch of each component returned, as objective_function / objective_function_jacobian hand it to
+    their caller: J_k of all components ('objective', shape (64,)) and grad J_k concatenated in component order, each in
+    the coefficient layout [nonmonotone | monotone] ('gradient').  Every rank reads its own components; one all-reduce
+    of the zero-padded vectors assembles the whole map."""
+    from ttt_b200 import binding as B
+    off = np.concatenate(([0], np.cumsum([len(c) for c in coefs])))
+    J, grad = np.zeros(len(coefs)), np.zeros(int(off[-1]))
+    for k in ks:
+        out = np.empty(1 + len(coefs[k]))
+        B.check(tm._lib.ttm_plan_get_out(tm._plans[k], B.dptr(out), out.size, tm._stream()))
+        G = tm._gram_nonmon(k)
+        if G is not None:                      # Gram mode: the kernel returned h, dJ/da = G a + h
+            m = G.shape[0]
+            out[1:1 + m] += G @ coefs[k][:m]
+        J[k], grad[off[k]:off[k + 1]] = out[0], out[1:]
+    if world > 1:
+        both = torch.from_numpy(np.concatenate((J, grad))).cuda()
+        dist.all_reduce(both)
+        both = both.cpu().numpy()
+        J, grad = both[:len(J)], both[len(J):]
+    return {'objective': J, 'gradient': grad}
+
+
 def multi_gpu_check(rank, world, dist, torch):
     """Sample-sharded evaluation (the K < #GPUs path of SURVEY 8(e): every rank holds N/world rows, (J, grad) are
     all-reduced) against the same evaluation on the whole ensemble held by one rank (the component-sharded layout)."""
@@ -651,6 +675,8 @@ def run_gpu(args):
     barrier()
     wall_value = time.perf_counter() - wall0
     t_local = float(sum(t_steps))
+    # read before the e2e leg below reuses the plans
+    outputs = step_outputs(tm, mine, coefs, world, dist, torch) if args.dump_outputs else None
 
     # ---- e2e: through the public class API with host coefficient vectors in, host (J, grad) out
     rng = np.random.default_rng(1)
@@ -850,6 +876,10 @@ def run_gpu(args):
             line['inverse_map'] = inv
             if 'parity_max_abs' in inv:
                 line.setdefault('parity', {})['inverse_max_abs'] = inv['parity_max_abs']
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
         sys.stdout.flush()
         os.dup2(saved_stdout, 1)
         print(json.dumps(line))
@@ -871,7 +901,14 @@ def main():
     ap.add_argument('--no-fit', action='store_true', help='skip the end-to-end optimize() of the C4 map')
     ap.add_argument('--streams', type=int, default=2, help='CUDA streams the evaluations of a step are issued on')
     ap.add_argument('--bps', type=int, default=2, help='resident blocks per SM of one launch (x streams = blocks per SM)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed to DIR as float64 .npy files: '
+                         'objective.npy (J_k, k = 0..63) and gradient.npy (grad J_k in component order)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU run')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -15,7 +15,8 @@ compare against:
   headline_sep_fit_<D>.npz  separable C5-pattern fit (QR path, tm.py:2966-2975 + L-BFGS-B :3108) at D=64 and D=128,
                             N=4000 (m_non up to 382): coefficients + map() head
   headline_c5_inverse.npz   C5 at D=256, E=128 conditioning columns: table and bisection inverse_map
-                            (tm.py:3639-4084) at seeded coefficients
+                            (tm.py:3639-4084) at seeded coefficients: the solved columns X[:, E:] of a fixed
+                            sample of the rows, with the row indices (all of it would pass 1 MB)
 
 The reference's own process pool (workers = cpu_count, tm.py:2789-2845) is used for the fits.
 """
@@ -109,11 +110,14 @@ def c5_inverse():
     rng = np.random.default_rng(C5_INV['seed'])
     Xstar = synthetic_samples(n_tab, D, seed=C5_INV['seed'] + 1)[:, :E].copy()
     Z = rng.standard_normal((n_tab, D - E))
-    out = {}
+    pick = np.random.default_rng(0)
+    rt = np.sort(pick.choice(n_tab, 200, replace=False))
+    rb = np.sort(pick.choice(n_bis, 80, replace=False))
+    out = {'rows_table': rt, 'rows_bisect': rb}
     tm.alternate_root_finding = True
-    out['inverse_table'] = tm.inverse_map(copy.copy(Z), X_star=copy.copy(Xstar))
+    out['inverse_table'] = tm.inverse_map(copy.copy(Z), X_star=copy.copy(Xstar))[rt, E:]
     tm.alternate_root_finding = False
-    out['inverse_bisect'] = tm.inverse_map(copy.copy(Z[:n_bis]), X_star=copy.copy(Xstar[:n_bis]))
+    out['inverse_bisect'] = tm.inverse_map(copy.copy(Z[:n_bis]), X_star=copy.copy(Xstar[:n_bis]))[rb, E:]
     save('headline_c5_inverse', out)
 
 

@@ -14,7 +14,8 @@ spec = importlib.util.spec_from_file_location(
 P = importlib.util.module_from_spec(spec)
 spec.loader.exec_module(P)
 
-EX01_PICKLE = '/root/reference/Examples A - spiral distribution/Example 01 - full map/dict_coeffs_order=10.p'
+# the coefficients of the reference's Example 01 pickle (dict_coeffs_order=10.p), per component [nonmonotone | monotone]
+EX01_KNOWN_ANSWER = os.path.join(HERE, 'golden', 'ex01_known_answer.npz')
 
 
 class FakeMap:
@@ -51,13 +52,23 @@ def test_shape_mismatch_is_an_error(tmp_path):
         P.load_coefficients(FakeMap([(3, 1), (5, 7)]), path)
 
 
-@pytest.mark.skipif(not os.path.exists(EX01_PICKLE), reason='reference checkout not present (GPU box)')
-def test_reads_the_pickle_shipped_with_example_01():
-    d = pickle.load(open(EX01_PICKLE, 'rb'))
+def test_reads_the_pickle_shipped_with_example_01(tmp_path):
+    """Example 01's shipped coefficients, pickled the way example_01.py:215-224 writes them."""
+    ka = np.load(EX01_KNOWN_ANSWER)
+    d = {'coeffs_mon': [], 'coeffs_nonmon': []}
+    for k in range(2):
+        c, div = ka['full_coeffs_%d' % k], int(ka['full_div_%d' % k])
+        d['coeffs_nonmon'].append(c[:div])
+        d['coeffs_mon'].append(c[div:])
+    path = tmp_path / 'dict_coeffs_order=10.p'
+    with open(path, 'wb') as f:
+        pickle.dump(d, f)
     tm = FakeMap([(len(m), len(n)) for m, n in zip(d['coeffs_mon'], d['coeffs_nonmon'])])
-    P.load_coefficients(tm, EX01_PICKLE)
+    P.load_coefficients(tm, path)
     assert tm.D == 2 and len(tm.coeffs_mon[1]) == 55 and len(tm.coeffs_nonmon[1]) == 11
-    assert np.array_equal(tm.coeffs_mon[1], np.asarray(d['coeffs_mon'][1]))
+    for k in range(2):
+        assert np.array_equal(tm.coeffs_mon[k], d['coeffs_mon'][k])
+        assert np.array_equal(tm.coeffs_nonmon[k], d['coeffs_nonmon'][k])
 
 
 def test_chronicle_layout(tmp_path):

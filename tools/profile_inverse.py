@@ -1,6 +1,7 @@
 import os, sys, time, json
 import numpy as np
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import torch
 from cases import synthetic_samples, c5_terms
 from transport_map import transport_map
