@@ -36,6 +36,10 @@ typedef struct ttm_plan ttm_plan; /* one compiled map component (term tables + w
 #define TTM_ERR_ARG -2
 #define TTM_ERR_LIMIT -3 /* plan exceeds a compiled limit (order > 20, > 8 special inner terms) */
 
+/* element type of a caller's row-major sample array (the *_ld entry points); float32 is widened on load */
+#define TTM_DTYPE_F64 0
+#define TTM_DTYPE_F32 1
+
 #define TTM_WHICH_NONMON 0
 #define TTM_WHICH_MON 1
 #define TTM_WHICH_DMON 2
@@ -87,6 +91,14 @@ int ttm_colstats(ttm_ctx* ctx, const double* X, int64_t N, int D, double* mean, 
 /* Xt[v*ld + i] = (X[i*D + v] - mean[v]) / std[v]   (mean == NULL: plain transpose)              */
 int ttm_standardize_transpose(ttm_ctx* ctx, const double* X, int64_t N, int D, const double* mean,
                               const double* std, double* Xt, int64_t ld, void* stream);
+/* The same two for a caller's row-major array read in place: row i at (char*)X + i*ldx*elemsize, ldx >= D (e.g. a
+ * column slice X[:, a:b] of a wider array), elements of type `dtype` (TTM_DTYPE_F64 / TTM_DTYPE_F32, widened to double
+ * as they are loaded, so a float32 array gives the bits its float64 copy gives).  The entry points above are these with
+ * (TTM_DTYPE_F64, ldx = D).  TTM_ERR_ARG on ldx < D or an unknown dtype. */
+int ttm_colstats_ld(ttm_ctx* ctx, const void* X, int dtype, int64_t ldx, int64_t N, int D, double* mean, double* std,
+                    double* scratch, void* stream);
+int ttm_standardize_transpose_ld(ttm_ctx* ctx, const void* X, int dtype, int64_t ldx, int64_t N, int D,
+                                 const double* mean, const double* std, double* Xt, int64_t ld, void* stream);
 /* X[i*ldx + v] = Xt[v*ld + i] * std[v] + mean[v]   (un-standardise, tm.py:3700-3704; NULL: transpose) */
 int ttm_transpose_back(ttm_ctx* ctx, const double* Xt, int64_t ld, int64_t N, int D, const double* mean,
                        const double* std, double* X, int64_t ldx, void* stream);
@@ -146,6 +158,10 @@ int ttm_density_finish(ttm_ctx* ctx, const double* acc, const double* log_target
 int ttm_map_fused(ttm_ctx* ctx, ttm_plan* const* host_plans, int D, const double* host_sigma, const double* X, int64_t n,
                   int Dtot, const double* mean, const double* std, const double* log_target, int mode, double* Z,
                   double* out, void* stream);
+/* the same on a caller's row-major array read in place (row stride ldx >= Dtot, dtype as for ttm_colstats_ld) */
+int ttm_map_fused_ld(ttm_ctx* ctx, ttm_plan* const* host_plans, int D, const double* host_sigma, const void* X, int dtype,
+                     int64_t ldx, int64_t n, int Dtot, const double* mean, const double* std, const double* log_target,
+                     int mode, double* Z, double* out, void* stream);
 
 /* ---- K-gram (FP64 tensor-core DMMA) ----------------------------------------------------------
  * replaces: the dense contractions of worker_task_monotone, tm.py:2966-2975 (QR / A_sqrt) and

@@ -17,6 +17,8 @@ c_void_p, c_int, c_int64, c_double = ctypes.c_void_p, ctypes.c_int, ctypes.c_int
 _dp = ctypes.POINTER(c_double)
 _ip = ctypes.POINTER(ctypes.c_int32)
 
+TTM_DTYPE_F64, TTM_DTYPE_F32 = 0, 1     # include/ttm.h: element type of the *_ld entry points
+
 _lib = None
 
 
@@ -48,6 +50,10 @@ def lib():
             'ttm_colstats': [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
             'ttm_standardize_transpose': [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int64,
                                           c_void_p],
+            'ttm_colstats_ld': [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p,
+                                c_void_p],
+            'ttm_standardize_transpose_ld': [c_void_p, c_void_p, c_int, c_int64, c_int64, c_int, c_void_p, c_void_p,
+                                             c_void_p, c_int64, c_void_p],
             'ttm_transpose_back': [c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int64,
                                    c_void_p],
             'ttm_basis_eval': [c_void_p, c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p],
@@ -60,6 +66,8 @@ def lib():
             'ttm_sep_eval': [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p],
             'ttm_map_fused': [c_void_p, ctypes.POINTER(c_void_p), c_int, _dp, c_void_p, c_int64, c_int, c_void_p, c_void_p,
                               c_void_p, c_int, c_void_p, c_void_p, c_void_p],
+            'ttm_map_fused_ld': [c_void_p, ctypes.POINTER(c_void_p), c_int, _dp, c_void_p, c_int, c_int64, c_int64, c_int,
+                                 c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
             'ttm_gram': [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p],
             'ttm_gram_tail': [c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p],
             'ttm_sep_objgrad': [c_void_p, c_void_p, c_int64, c_int64, _dp, _dp, c_void_p],

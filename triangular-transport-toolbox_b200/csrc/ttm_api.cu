@@ -282,19 +282,33 @@ int ttm_plan_destroy(ttm_plan* p) {
     return TTM_OK;
 }
 
-int ttm_colstats(ttm_ctx* c, const double* X, int64_t N, int D, double* mean, double* sd, double* scratch, void* stream) {
-    if (!c || !X || N <= 0 || D <= 0) return fail(TTM_ERR_ARG, "ttm_colstats: bad arguments");
+static bool known_dtype(int dtype) { return dtype == TTM_DTYPE_F64 || dtype == TTM_DTYPE_F32; }
+
+int ttm_colstats_ld(ttm_ctx* c, const void* X, int dtype, int64_t ldx, int64_t N, int D, double* mean, double* sd,
+                    double* scratch, void* stream) {
+    if (!c || !X || N <= 0 || D <= 0 || ldx < D || !known_dtype(dtype))
+        return fail(TTM_ERR_ARG, "ttm_colstats_ld: bad arguments");
     CK(cudaSetDevice(c->device));
-    CK(ttm_launch_colstats(X, N, D, mean, sd, scratch, c->sm_count, (cudaStream_t)stream));
+    CK(ttm_launch_colstats(X, dtype, ldx, N, D, mean, sd, scratch, c->sm_count, (cudaStream_t)stream));
+    return TTM_OK;
+}
+
+int ttm_colstats(ttm_ctx* c, const double* X, int64_t N, int D, double* mean, double* sd, double* scratch, void* stream) {
+    return ttm_colstats_ld(c, X, TTM_DTYPE_F64, D, N, D, mean, sd, scratch, stream);
+}
+
+int ttm_standardize_transpose_ld(ttm_ctx* c, const void* X, int dtype, int64_t ldx, int64_t N, int D, const double* mean,
+                                 const double* sd, double* Xt, int64_t ld, void* stream) {
+    if (!c || !X || !Xt || N <= 0 || D <= 0 || ld < N || ldx < D || !known_dtype(dtype))
+        return fail(TTM_ERR_ARG, "ttm_standardize_transpose_ld: bad arguments");
+    CK(cudaSetDevice(c->device));
+    CK(ttm_launch_standardize_transpose(X, dtype, ldx, N, D, mean, sd, Xt, ld, (cudaStream_t)stream));
     return TTM_OK;
 }
 
 int ttm_standardize_transpose(ttm_ctx* c, const double* X, int64_t N, int D, const double* mean, const double* sd,
                               double* Xt, int64_t ld, void* stream) {
-    if (!c || !X || !Xt || N <= 0 || D <= 0 || ld < N) return fail(TTM_ERR_ARG, "ttm_standardize_transpose: bad arguments");
-    CK(cudaSetDevice(c->device));
-    CK(ttm_launch_standardize_transpose(X, N, D, mean, sd, Xt, ld, (cudaStream_t)stream));
-    return TTM_OK;
+    return ttm_standardize_transpose_ld(c, X, TTM_DTYPE_F64, D, N, D, mean, sd, Xt, ld, stream);
 }
 
 int ttm_transpose_back(ttm_ctx* c, const double* Xt, int64_t ld, int64_t N, int D, const double* mean, const double* sd,
@@ -466,11 +480,11 @@ int ttm_density_finish(ttm_ctx* c, const double* acc, const double* log_target, 
     return TTM_OK;
 }
 
-int ttm_map_fused(ttm_ctx* c, ttm_plan* const* host_plans, int D, const double* host_sigma, const double* X, int64_t n,
-                  int Dtot, const double* mean, const double* sd, const double* log_target, int mode, double* Z, double* out,
-                  void* stream) {
+int ttm_map_fused_ld(ttm_ctx* c, ttm_plan* const* host_plans, int D, const double* host_sigma, const void* X, int dtype,
+                     int64_t ldx, int64_t n, int Dtot, const double* mean, const double* sd, const double* log_target,
+                     int mode, double* Z, double* out, void* stream) {
     if (!c || !host_plans || D <= 0 || !X || n <= 0 || Dtot <= 0 || mode < 0 || mode > 2 || (mode != 2 && (!out || !host_sigma)) ||
-        (mode == 2 && !Z) || ((mean == nullptr) != (sd == nullptr)))
+        (mode == 2 && !Z) || ((mean == nullptr) != (sd == nullptr)) || ldx < Dtot || !known_dtype(dtype))
         return fail(TTM_ERR_ARG, "ttm_map_fused: bad arguments");
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -493,12 +507,20 @@ int ttm_map_fused(ttm_ctx* c, ttm_plan* const* host_plans, int D, const double* 
     CK(cudaMemcpyAsync(c->d_fused, c->h_fused, D * sizeof(FusedComp), cudaMemcpyHostToDevice, st));
     CK(cudaEventRecord(c->ev_fused, st));
     FusedMapArgs a;
-    a.comps = c->d_fused; a.D = D; a.Dtot = Dtot; a.X = X; a.n = n; a.mean = mean; a.sd = sd; a.logt = log_target;
+    a.comps = c->d_fused; a.D = D; a.Dtot = Dtot; a.X = X; a.dtype = dtype; a.ldx = ldx; a.n = n;
+    a.mean = mean; a.sd = sd; a.logt = log_target;
     a.mode = mode; a.Z = Z; a.out = out;
     cudaError_t e = ttm_launch_map_fused(a, st);
     if (e == cudaErrorInvalidValue) return fail(TTM_ERR_LIMIT, "ttm_map_fused: too many columns for one shared-memory tile");
     CK(e);
     return TTM_OK;
+}
+
+int ttm_map_fused(ttm_ctx* c, ttm_plan* const* host_plans, int D, const double* host_sigma, const double* X, int64_t n,
+                  int Dtot, const double* mean, const double* sd, const double* log_target, int mode, double* Z, double* out,
+                  void* stream) {
+    return ttm_map_fused_ld(c, host_plans, D, host_sigma, X, TTM_DTYPE_F64, Dtot, n, Dtot, mean, sd, log_target, mode, Z,
+                            out, stream);
 }
 
 int ttm_gram(ttm_plan* p, const double* Xt, int64_t ld, int64_t N, double* G, double* scratch, int64_t scratch_doubles,

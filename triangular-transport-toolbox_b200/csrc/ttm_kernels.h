@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/ttm.h"
 #include "ttm_common.cuh"
 
 struct ObjArgs {
@@ -46,11 +47,13 @@ cudaError_t ttm_launch_objgrad(const ObjArgs& a, bool grad, int sm_count, cudaSt
 // tile kernel; cudaErrorNotSupported if the plan is outside its class
 cudaError_t ttm_launch_objgrad_tile(const ObjArgs& a, bool grad, int sm_count, cudaStream_t st);
 
-// column statistics + standardise + transpose (reference: standardize, transport_map.py:750-787)
-cudaError_t ttm_launch_colstats(const double* X, int64_t N, int D, double* mean, double* std, double* scratch,
-                                int sm_count, cudaStream_t st);
-cudaError_t ttm_launch_standardize_transpose(const double* X, int64_t N, int D, const double* mean,
-                                             const double* std, double* Xt, int64_t ld, cudaStream_t st);
+// column statistics + standardise + transpose (reference: standardize, transport_map.py:750-787).
+// X: row-major (N, >= D) samples of dtype TTM_DTYPE_F64 / TTM_DTYPE_F32 with row stride ldx
+cudaError_t ttm_launch_colstats(const void* X, int dtype, int64_t ldx, int64_t N, int D, double* mean, double* std,
+                                double* scratch, int sm_count, cudaStream_t st);
+cudaError_t ttm_launch_standardize_transpose(const void* X, int dtype, int64_t ldx, int64_t N, int D,
+                                             const double* mean, const double* std, double* Xt, int64_t ld,
+                                             cudaStream_t st);
 cudaError_t ttm_launch_transpose_back(const double* Xt, int64_t ld, int64_t N, int D, const double* mean,
                                       const double* std, double* X, int64_t ldx, int col0, cudaStream_t st);
 
@@ -79,7 +82,9 @@ struct FusedComp {
 struct FusedMapArgs {
     const FusedComp* comps;  // device [D]
     int D, Dtot;
-    const double* X;         // device row-major (n, Dtot) UNstandardised samples
+    const void* X;           // device row-major (n, >= Dtot) UNstandardised samples, row stride ldx
+    int dtype;               // TTM_DTYPE_F64 / TTM_DTYPE_F32 (widened on load)
+    int64_t ldx;
     int64_t n;
     const double* mean;      // device [Dtot] or NULL (no standardisation)
     const double* sd;

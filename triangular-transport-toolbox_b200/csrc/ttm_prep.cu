@@ -11,8 +11,9 @@ namespace {
 constexpr int T_STAT = 256;
 
 // pass 0: per-block column sums of x;  pass 1: per-block column sums of (x-mean)^2
-template <int PASS>
-__global__ void __launch_bounds__(T_STAT) colsum_kernel(const double* __restrict__ X, int64_t N, int D, int c0, int Dc,
+// X: row-major rows of T (double or float, widened on load) with row stride ldx >= D
+template <int PASS, typename T>
+__global__ void __launch_bounds__(T_STAT) colsum_kernel(const T* __restrict__ X, int64_t ldx, int64_t N, int c0, int Dc,
                                                         const double* __restrict__ mean, double* __restrict__ part) {
     __shared__ double red[T_STAT];
     const int lanes = T_STAT / Dc;            // rows handled concurrently by one block
@@ -21,7 +22,7 @@ __global__ void __launch_bounds__(T_STAT) colsum_kernel(const double* __restrict
     if (rl < lanes) {
         const double mu = PASS ? mean[c0 + d] : 0.0;
         for (int64_t i = (int64_t)blockIdx.x * lanes + rl; i < N; i += (int64_t)gridDim.x * lanes) {
-            const double v = X[i * D + c0 + d] - mu;
+            const double v = (double)X[i * ldx + c0 + d] - mu;
             acc += PASS ? v * v : v;
         }
     }
@@ -45,8 +46,9 @@ __global__ void colsum_final_kernel(const double* __restrict__ part, int nblocks
     out[c0 + d] = PASS ? sqrt(s) : s;
 }
 
-// Xt[d*ld + i] = (X[i*D + d] - mean[d]) / std[d]     (32x32 smem tile transpose)
-__global__ void __launch_bounds__(256) std_transpose_kernel(const double* __restrict__ X, int64_t N, int D,
+// Xt[d*ld + i] = (X[i*ldx + d] - mean[d]) / std[d]     (32x32 smem tile transpose; T widened on load)
+template <typename T>
+__global__ void __launch_bounds__(256) std_transpose_kernel(const T* __restrict__ X, int64_t ldx, int64_t N, int D,
                                                             const double* __restrict__ mean,
                                                             const double* __restrict__ sd, double* __restrict__ Xt,
                                                             int64_t ld) {
@@ -59,7 +61,7 @@ __global__ void __launch_bounds__(256) std_transpose_kernel(const double* __rest
         const int64_t i = i0 + ty + 8 * k;
         const int d = d0 + tx;
         if (i < N && d < D) {
-            double v = X[i * D + d];
+            double v = (double)X[i * ldx + d];
             if (mean) v = (v - mean[d]) / sd[d];
             tile[ty + 8 * k][tx] = v;
         }
@@ -244,8 +246,9 @@ __global__ void fp64_peak_kernel(double* sink, int iters) {
 
 }  // namespace
 
-cudaError_t ttm_launch_colstats(const double* X, int64_t N, int D, double* mean, double* sd, double* scratch,
-                                int sm_count, cudaStream_t st) {
+template <typename T>
+static cudaError_t launch_colstats(const T* X, int64_t ldx, int64_t N, int D, double* mean, double* sd, double* scratch,
+                                   int sm_count, cudaStream_t st) {
     // scratch: >= sm_count*4*256 doubles
     for (int c0 = 0; c0 < D; c0 += T_STAT) {
         const int Dc = min(T_STAT, D - c0);
@@ -253,18 +256,28 @@ cudaError_t ttm_launch_colstats(const double* X, int64_t N, int D, double* mean,
         int64_t grid = (N + lanes - 1) / lanes;
         if (grid > (int64_t)sm_count * 4) grid = (int64_t)sm_count * 4;
         if (grid < 1) grid = 1;
-        colsum_kernel<0><<<(int)grid, T_STAT, 0, st>>>(X, N, D, c0, Dc, nullptr, scratch);
+        colsum_kernel<0, T><<<(int)grid, T_STAT, 0, st>>>(X, ldx, N, c0, Dc, nullptr, scratch);
         colsum_final_kernel<0><<<(Dc + 127) / 128, 128, 0, st>>>(scratch, (int)grid, Dc, c0, N, mean);
-        colsum_kernel<1><<<(int)grid, T_STAT, 0, st>>>(X, N, D, c0, Dc, mean, scratch);
+        colsum_kernel<1, T><<<(int)grid, T_STAT, 0, st>>>(X, ldx, N, c0, Dc, mean, scratch);
         colsum_final_kernel<1><<<(Dc + 127) / 128, 128, 0, st>>>(scratch, (int)grid, Dc, c0, N, sd);
     }
     return cudaGetLastError();
 }
 
-cudaError_t ttm_launch_standardize_transpose(const double* X, int64_t N, int D, const double* mean, const double* sd,
-                                             double* Xt, int64_t ld, cudaStream_t st) {
+cudaError_t ttm_launch_colstats(const void* X, int dtype, int64_t ldx, int64_t N, int D, double* mean, double* sd,
+                                double* scratch, int sm_count, cudaStream_t st) {
+    if (dtype == TTM_DTYPE_F32)
+        return launch_colstats(static_cast<const float*>(X), ldx, N, D, mean, sd, scratch, sm_count, st);
+    return launch_colstats(static_cast<const double*>(X), ldx, N, D, mean, sd, scratch, sm_count, st);
+}
+
+cudaError_t ttm_launch_standardize_transpose(const void* X, int dtype, int64_t ldx, int64_t N, int D, const double* mean,
+                                             const double* sd, double* Xt, int64_t ld, cudaStream_t st) {
     dim3 grid((unsigned)((N + 31) / 32), (unsigned)((D + 31) / 32));
-    std_transpose_kernel<<<grid, 256, 0, st>>>(X, N, D, mean, sd, Xt, ld);
+    if (dtype == TTM_DTYPE_F32)
+        std_transpose_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(X), ldx, N, D, mean, sd, Xt, ld);
+    else
+        std_transpose_kernel<double><<<grid, 256, 0, st>>>(static_cast<const double*>(X), ldx, N, D, mean, sd, Xt, ld);
     return cudaGetLastError();
 }
 

@@ -251,7 +251,7 @@ cudaError_t ttm_launch_sepobj_batch(const SepBatchItem* d_items, const SepBatchL
 
 // -------------------------------------------------------------------------------------------------
 // K-map-fused / K-pullback (small separable maps): ALL components of the map on a tile of samples in one launch,
-// reading the caller's row-major samples directly (standardisation on the fly) and writing row-major Z and/or the
+// reading the caller's row-major samples directly (float64 or float32, any row stride; standardisation on the fly) and writing row-major Z and/or the
 // density -- no transposes, no per-component launches, no S / dS / accumulator round trips through HBM.
 //   map                 tm.py:2391-2437 (separable arm of s, :2550-2558)
 //   pullback density    tm.py:2646-2712:  exp( sum_k [-S_k^2/2 - log(2 pi)/2] + sum_k log(dS_k / sigma_k) )
@@ -265,6 +265,7 @@ namespace {
 
 constexpr int T_FUSE = 128;
 
+template <typename T>
 __global__ void __launch_bounds__(T_FUSE) map_fused_kernel(const FusedMapArgs a) {
     extern __shared__ double sm[];
     const int ldt = T_FUSE + 1;
@@ -273,9 +274,10 @@ __global__ void __launch_bounds__(T_FUSE) map_fused_kernel(const FusedMapArgs a)
     const int tid = threadIdx.x;
     const int64_t base = (int64_t)blockIdx.x * T_FUSE;
     const int rows = (int)min((int64_t)T_FUSE, a.n - base);
+    const T* __restrict__ X = static_cast<const T*>(a.X);
     for (int e = tid; e < rows * a.Dtot; e += T_FUSE) {
         const int r = e / a.Dtot, v = e - r * a.Dtot;
-        const double x = a.X[(base + r) * a.Dtot + v];
+        const double x = (double)X[(base + r) * a.ldx + v];
         t_raw[v * ldt + r] = x;
         t_std[v * ldt + r] = a.mean ? (x - a.mean[v]) / a.sd[v] : x;
     }
@@ -305,14 +307,19 @@ __global__ void __launch_bounds__(T_FUSE) map_fused_kernel(const FusedMapArgs a)
 
 }  // namespace
 
+template <typename T>
+static cudaError_t launch_map_fused(const FusedMapArgs& a, size_t smem, cudaStream_t st) {
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(map_fused_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    map_fused_kernel<T><<<(unsigned)((a.n + T_FUSE - 1) / T_FUSE), T_FUSE, smem, st>>>(a);
+    return cudaGetLastError();
+}
+
 cudaError_t ttm_launch_map_fused(const FusedMapArgs& a, cudaStream_t st) {
     if (a.n == 0) return cudaSuccess;
     const size_t smem = sizeof(double) * (size_t)(2 * a.Dtot * (T_FUSE + 1));
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(map_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-    }
-    map_fused_kernel<<<(unsigned)((a.n + T_FUSE - 1) / T_FUSE), T_FUSE, smem, st>>>(a);
-    return cudaGetLastError();
+    return a.dtype == TTM_DTYPE_F32 ? launch_map_fused<float>(a, smem, st) : launch_map_fused<double>(a, smem, st);
 }

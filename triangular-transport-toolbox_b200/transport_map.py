@@ -35,6 +35,25 @@ def _torch():
     return torch
 
 
+_SHAPE_MSG = ('X should be a two-dimensional array of shape (N,D), N = number of samples, '
+              'D = number of dimensions. Current shape of X is ')
+
+
+class _DevSamples:
+    """A CUDA-tensor sample argument as the *_ld kernels read it in place: n rows of d values, row stride `ld`
+    elements, float64 or float32 (`code`: B.TTM_DTYPE_*).  `t` is the tensor (it keeps the storage alive)."""
+    __slots__ = ('t', 'n', 'd', 'ld', 'code')
+
+    def __init__(self, t, n, d, ld, code):
+        self.t, self.n, self.d, self.ld, self.code = t, n, d, ld, code
+
+    ndim = 2
+
+    @property
+    def shape(self):
+        return (self.n, self.d)
+
+
 class _LazyList:
     """List-like view whose items are computed on first access (Psi_mon, Psi_nonmon, der_Psi_mon)."""
 
@@ -226,16 +245,52 @@ class transport_map():
         a = np.ascontiguousarray(a, dtype=np.float64)
         return self._torch.from_numpy(a).to(self._device, non_blocking=False)
 
-    def _to_colmajor(self, X_host, mean=None, std=None):
-        """row-major host (n, d) -> device column-major (d, n), optionally standardised with (mean, std)."""
-        n, d = X_host.shape
-        Xd = self._upload(X_host)
-        Xt = self._empty(d, n)
+    def _samples(self, X, ncol=None):
+        """Classify a sample-array argument.  numpy arrays, lists and CPU tensors -> float64 numpy array (the host path).
+        A CUDA tensor -> _DevSamples, checked before any launch (2-D, `ncol` columns if given, on this map's device):
+        float64 / float32 with unit column stride and a row stride >= d are read in place (column views such as
+        Xe[:, skip:]); any other dtype or layout is converted once on the device, as np.asarray(X, float64) converts
+        on the host."""
+        torch = self._torch
+        if isinstance(X, _DevSamples):
+            return X
+        if not (isinstance(X, torch.Tensor) and X.is_cuda):
+            return np.asarray(X, dtype=np.float64)
+        if X.ndim != 2:
+            raise ValueError(_SHAPE_MSG + str(tuple(X.shape)))
+        if X.device != self._device:
+            raise ValueError('the tensor is on %s; this map runs on %s' % (X.device, self._device))
+        n, d = X.shape
+        if ncol is not None and d != ncol:
+            raise ValueError('operands could not be broadcast together: %d columns vs %d' % (d, ncol))
+        if (X.dtype not in (torch.float64, torch.float32) or (d > 1 and X.stride(1) != 1)
+                or (n > 1 and X.stride(0) < d)):
+            X = X.to(torch.float64).contiguous()
+        return _DevSamples(X, n, d, X.stride(0) if n > 1 else max(d, 1),
+                           B.TTM_DTYPE_F32 if X.dtype == torch.float32 else B.TTM_DTYPE_F64)
+
+    def _on_device(self, X):
+        """_DevSamples of a host float64 (n, d) array (uploaded contiguous) or of a _DevSamples (itself)."""
+        if isinstance(X, _DevSamples):
+            return X
+        t = self._upload(X)
+        n, d = t.shape
+        return _DevSamples(t, n, d, d, B.TTM_DTYPE_F64)
+
+    def _to_colmajor(self, X, mean=None, std=None, out=None):
+        """row-major (n, d) samples (host array or _DevSamples) -> device column-major (d, n), optionally standardised
+        with (mean, std); written to rows [0, d) of `out` (ld = out.shape[1]) instead of a new tensor if given."""
+        S = self._on_device(X)
+        Xt = self._empty(S.d, S.n) if out is None else out
         mp = B.c_void_p(mean.data_ptr()) if mean is not None else None
         sp = B.c_void_p(std.data_ptr()) if std is not None else None
-        B.check(self._lib.ttm_standardize_transpose(self._ctx, B.c_void_p(Xd.data_ptr()), n, d, mp, sp,
-                                                    B.c_void_p(Xt.data_ptr()), n, self._stream()))
+        B.check(self._lib.ttm_standardize_transpose_ld(self._ctx, B.c_void_p(S.t.data_ptr()), S.code, S.ld, S.n, S.d,
+                                                       mp, sp, B.c_void_p(Xt.data_ptr()), Xt.shape[1], self._stream()))
         return Xt
+
+    def _result(self, t, dev):
+        """Output step: the device tensor itself for a CUDA-tensor call (dev), else downloaded to numpy."""
+        return t if dev else self._download(t)
 
     def _download(self, t):
         """Device tensor -> numpy.  Large results go through a pinned staging tensor from torch's caching host
@@ -246,23 +301,24 @@ class transport_map():
         host.copy_(t, non_blocking=False)
         return host.numpy()
 
-    def _to_rowmajor(self, Xt, n, d, mean=None, std=None):
-        """device column-major (d, ld>=n) -> host row-major (n, d), optionally un-standardised."""
+    def _to_rowmajor(self, Xt, n, d, mean=None, std=None, dev=False):
+        """device column-major (d, ld>=n) -> row-major (n, d), optionally un-standardised: host array, or the
+        device tensor if dev."""
         out = self._empty(n, d)
         mp = B.c_void_p(mean.data_ptr()) if mean is not None else None
         sp = B.c_void_p(std.data_ptr()) if std is not None else None
         B.check(self._lib.ttm_transpose_back(self._ctx, B.c_void_p(Xt.data_ptr()), Xt.shape[1], n, d, mp, sp,
                                              B.c_void_p(out.data_ptr()), d, self._stream()))
-        return self._download(out)
+        return self._result(out, dev)
 
     def _load_samples(self, X):
-        """Upload the training ensemble, standardise it on the device (tm.py:750-787) and keep the
-        column-major copy resident."""
+        """Upload the training ensemble (or read a CUDA tensor in place), standardise it on the device
+        (tm.py:750-787) and keep the column-major copy resident.  Quantile standardisation downloads the samples
+        for numpy's order statistics (setup, once per reset)."""
         torch = self._torch
-        X = np.asarray(X, dtype=np.float64)
+        X = self._samples(X)
         if X.ndim != 2:
-            raise Exception('X should be a two-dimensional array of shape (N,D), N = number of samples, '
-                            'D = number of dimensions. Current shape of X is ' + str(X.shape))
+            raise Exception(_SHAPE_MSG + str(X.shape))
         n, d = X.shape
         self._N, self._Dtot = n, d
         self._N_global = n
@@ -279,12 +335,11 @@ class transport_map():
             return
         mode = self.standardization.lower()
         if mode == 'standard':
-            Xd = self._upload(X)
+            Xd = self._on_device(X)
             self._mean_d, self._std_d = self._empty(d), self._empty(d)
-            B.check(self._lib.ttm_colstats(self._ctx, B.c_void_p(Xd.data_ptr()), n, d,
-                                           B.c_void_p(self._mean_d.data_ptr()), B.c_void_p(self._std_d.data_ptr()),
-                                           B.c_void_p(self._scratch.data_ptr()), self._stream()))
-            self._Xt = self._empty(d, n)
+            B.check(self._lib.ttm_colstats_ld(self._ctx, B.c_void_p(Xd.t.data_ptr()), Xd.code, Xd.ld, n, d,
+                                              B.c_void_p(self._mean_d.data_ptr()), B.c_void_p(self._std_d.data_ptr()),
+                                              B.c_void_p(self._scratch.data_ptr()), self._stream()))
             if self._sharded:
                 # exact combination of the per-shard moments: one all-reduce of [n, n*mean, n*(var + mean^2)]
                 from .parallel import allreduce_sum
@@ -294,18 +349,16 @@ class transport_map():
                 gmu = tot[1:1 + d] / tot[0]
                 gsd = np.sqrt(np.maximum(tot[1 + d:] / tot[0] - gmu ** 2, 0.0))
                 self._mean_d, self._std_d = self._upload(gmu), self._upload(gsd)
-            B.check(self._lib.ttm_standardize_transpose(self._ctx, B.c_void_p(Xd.data_ptr()), n, d,
-                                                        B.c_void_p(self._mean_d.data_ptr()),
-                                                        B.c_void_p(self._std_d.data_ptr()),
-                                                        B.c_void_p(self._Xt.data_ptr()), n, self._stream()))
+            self._Xt = self._to_colmajor(Xd, self._mean_d, self._std_d)
             self.X_mean = self._mean_d.cpu().numpy()
             self.X_std = self._std_d.cpu().numpy()
             del Xd
         elif mode in ('quantile', 'quantiles'):
             # order statistics: host numpy (setup, not hot), exactly tm.py:775-778
-            self.X_mean = np.quantile(X, q=0.5, axis=0)
-            self.X_std = (np.quantile(X - self.X_mean, q=0.8413447460685429, axis=0) -
-                          np.quantile(X - self.X_mean, q=0.15865525393145707, axis=0)) / 2
+            Xh = X.t.to(torch.float64).cpu().numpy() if isinstance(X, _DevSamples) else X
+            self.X_mean = np.quantile(Xh, q=0.5, axis=0)
+            self.X_std = (np.quantile(Xh - self.X_mean, q=0.8413447460685429, axis=0) -
+                          np.quantile(Xh - self.X_mean, q=0.15865525393145707, axis=0)) / 2
             self._mean_d, self._std_d = self._upload(self.X_mean), self._upload(self.X_std)
             self._Xt = self._to_colmajor(X, self._mean_d, self._std_d)
         else:
@@ -321,7 +374,7 @@ class transport_map():
 
     @X.setter
     def X(self, value):
-        value = np.asarray(value, dtype=np.float64)
+        value = self._samples(value)
         self._Xt = self._to_colmajor(value)
         self._torch.cuda.current_stream(self._device).synchronize()
         self._N, self._Dtot = value.shape
@@ -543,9 +596,9 @@ class transport_map():
 
     def reset(self, X):
         """tm.py:710-748."""
+        X = self._samples(X)                       # a CUDA tensor of the wrong shape raises ValueError here
         if len(X.shape) != 2:
-            raise Exception('X should be a two-dimensional array of shape (N,D), N = number of samples, '
-                            'D = number of dimensions. Current shape of X is ' + str(X.shape))
+            raise Exception(_SHAPE_MSG + str(X.shape))
         self._load_samples(X)
         for k in range(self.D):
             self.coeffs_mon[k] = self.coeffs_mon[k] * 0 + self.coeffs_init
@@ -594,15 +647,19 @@ class transport_map():
             coeffs_mon = self.coeffs_mon[k]
         if coeffs_nonmon is None:
             coeffs_nonmon = self.coeffs_nonmon[k]
+        dev = False
         if x is None:
             Xt, n = self._Xt, self._N
         else:
-            x = np.asarray(x, dtype=np.float64)
+            x = self._samples(x, ncol=self._Dtot)
+            dev = isinstance(x, _DevSamples)
+            if dev and x.n == 0:
+                return self._empty(0)
             Xt, n = self._to_colmajor(x), x.shape[0]
         self._set_coeffs(k, coeffs_nonmon, coeffs_mon)
         out = self._empty(n)
         self._s_device(k, Xt, n, out)
-        return self._download(out)
+        return self._result(out, dev)
 
     # ------------------------------------------------------------------ fused small-map path (K-map-fused)
     def _fused_small(self):
@@ -615,29 +672,38 @@ class transport_map():
         return self._Dtot <= 64 and sum(p.m_non + p.m_mon + p.m_dmon for p in self._host_plans) <= 512
 
     def _map_fused(self, X, mode, sigma=None, log_target=None, want_Z=False):
-        """mode 0: pullback density (and Z), 1: pushforward density, 2: Z only; X row-major (n, Dtot) host array."""
-        X = np.ascontiguousarray(X, dtype=np.float64)
-        n = X.shape[0]
+        """mode 0: pullback density (and Z), 1: pushforward density, 2: Z only; X row-major (n, Dtot): host array
+        (results downloaded) or _DevSamples (results stay on the device); log_target: device vector or None."""
+        dev = isinstance(X, _DevSamples)
+        if X.ndim != 2 or X.shape[1] != self._Dtot:         # the kernel reads Dtot values per row
+            raise ValueError('operands could not be broadcast together: X has shape %s, the map has %d columns'
+                             % (tuple(X.shape), self._Dtot))
+        Xd = self._on_device(X if dev else np.ascontiguousarray(X))
+        n = Xd.n
         for k in range(self.D):
             self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
-        Xd = self._upload(X)
         Z = self._empty(n, self.D) if (want_Z or mode == 2) else None
         out = self._empty(n) if mode != 2 else None
-        lt = self._upload(log_target) if log_target is not None else None
         plans = (B.c_void_p * self.D)(*[h.value for h in self._plans])
         sg = np.ascontiguousarray(sigma, dtype=np.float64) if sigma is not None else None
         ptr = lambda t: B.c_void_p(t.data_ptr()) if t is not None else None
-        B.check(self._lib.ttm_map_fused(self._ctx, plans, self.D, B.dptr(sg) if sg is not None else None, ptr(Xd), n,
-                                        self._Dtot, ptr(self._mean_d), ptr(self._std_d), ptr(lt), mode, ptr(Z), ptr(out),
-                                        self._stream()))
-        return (self._download(Z) if Z is not None else None), (self._download(out) if out is not None else None)
+        B.check(self._lib.ttm_map_fused_ld(self._ctx, plans, self.D, B.dptr(sg) if sg is not None else None, ptr(Xd.t),
+                                           Xd.code, Xd.ld, n, self._Dtot, ptr(self._mean_d), ptr(self._std_d),
+                                           ptr(log_target), mode, ptr(Z), ptr(out), self._stream()))
+        return (self._result(Z, dev) if Z is not None else None), (self._result(out, dev) if out is not None else None)
 
     def map(self, X=None):
-        """Forward map target -> reference (tm.py:2391-2437)."""
+        """Forward map target -> reference (tm.py:2391-2437).  X: host array, or a CUDA tensor on the map's device
+        (the result is then a float64 CUDA tensor)."""
+        dev = False
+        if X is not None:
+            X = self._samples(X, ncol=self._Dtot)
+            dev = isinstance(X, _DevSamples)
+            if dev and X.n == 0:
+                return self._empty(0, self.D)
         if X is not None and self._fused_small():
             return self._map_fused(X, 2)[0]
         if X is not None and self.standardize_samples:
-            X = np.asarray(X, dtype=np.float64)
             Xt, n = self._to_colmajor(X, self._mean_d, self._std_d), X.shape[0]
         else:
             # NB the reference ignores a user-supplied X when standardize_samples is False (tm.py:2419-2422)
@@ -662,11 +728,11 @@ class transport_map():
                 a0 = float(sum(cat[q] for q in cs[cp[k]:cp[k + 1]]))
                 B.check(self._lib.ttm_sep_eval_base(self._plans[k], B.c_void_p(Xt.data_ptr()), Xt.shape[1], n,
                                                     B.c_void_p(base[k].data_ptr()), a0, B.c_void_p(Zt[k].data_ptr()), st))
-            return self._to_rowmajor(Zt, n, self.D)
+            return self._to_rowmajor(Zt, n, self.D, dev=dev)
         for k in range(self.D):
             self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
             self._s_device(k, Xt, n, Zt[k])
-        return self._to_rowmajor(Zt, n, self.D)
+        return self._to_rowmajor(Zt, n, self.D, dev=dev)
 
     def _map_gemm_static(self):
         """Packing indices of the forward map's GEMM operand (ttm_map_rect), or None when the map is outside its class:
@@ -1076,14 +1142,16 @@ class transport_map():
 
     # ================================================================== inverse map
     def inverse_map(self, Z, X_star=None):
-        """Inverse map reference -> target, optionally conditioned on X_star (tm.py:3639-3796)."""
-        Z = np.asarray(Z, dtype=np.float64)
+        """Inverse map reference -> target, optionally conditioned on X_star (tm.py:3639-3796).  Z: host array, or a
+        CUDA tensor on the map's device (the result is then a float64 CUDA tensor); X_star may be either kind."""
+        Z = self._samples(Z)
+        dev = isinstance(Z, _DevSamples)
         N = Z.shape[0]
         skip, D = self.skip_dimensions, self.D
         if X_star is None:
             ncol, comps, E = skip + D, [(k, k) for k in range(D)], 0
         else:
-            X_star = np.asarray(X_star, dtype=np.float64)
+            X_star = self._samples(X_star)
             if X_star.shape[-1] == skip:
                 ncol, comps, E = skip + D, [(k, k) for k in range(D)], skip
             elif skip == 0:
@@ -1093,16 +1161,24 @@ class transport_map():
                 raise UnboundLocalError("X_star has %d columns; expected skip_dimensions = %d" % (X_star.shape[-1], skip))
         if ncol != self._Dtot:
             raise ValueError("operands could not be broadcast together: %d columns vs %d" % (ncol, self._Dtot))
+        if dev and Z.shape[1] != len(comps):
+            raise ValueError("operands could not be broadcast together: %d columns vs %d" % (Z.shape[1], len(comps)))
+        if E > 0 and X_star.shape[0] != N:
+            raise ValueError("operands could not be broadcast together: %d samples in Z vs %d in X_star"
+                             % (N, X_star.shape[0]))
+        if dev and N == 0:
+            return self._empty(0, ncol - skip)
         torch = self._torch
         table_mode = self.alternate_root_finding and self.monotonicity.lower() == 'separable monotonicity'
-        if table_mode and N >= int(os.environ.get('TTM_INV_PIPELINE_MIN', 131072)):
+        # the pipeline hides host <-> device copies: device operands take the one-shot path (bit-identical)
+        if (table_mode and not dev and not isinstance(X_star, _DevSamples)
+                and N >= int(os.environ.get('TTM_INV_PIPELINE_MIN', 131072))):
             return self._inverse_map_pipelined(Z, X_star, E, ncol, comps)
         Xw = torch.zeros(ncol, N, dtype=torch.float64, device=self._device)
         if E > 0:
             std = self.standardize_samples
-            Xs = self._to_colmajor(X_star, self._mean_d[:E].contiguous() if std else None,
-                                   self._std_d[:E].contiguous() if std else None)
-            Xw[:E] = Xs
+            self._to_colmajor(X_star, self._mean_d[:E].contiguous() if std else None,
+                              self._std_d[:E].contiguous() if std else None, out=Xw)
         Zt = self._to_colmajor(Z)
         fused = self._inverse_fused_setup(comps) if table_mode else None
         if fused is not None:
@@ -1116,9 +1192,9 @@ class transport_map():
                 self._root_search_bisection(k, Xw, N, Zt[i])
         if self.standardize_samples:
             Xout = self._to_rowmajor(Xw[skip:], N, ncol - skip, self._mean_d[skip:].contiguous(),
-                                     self._std_d[skip:].contiguous())
+                                     self._std_d[skip:].contiguous(), dev=dev)
         else:
-            Xout = self._to_rowmajor(Xw[skip:], N, ncol - skip)
+            Xout = self._to_rowmajor(Xw[skip:], N, ncol - skip, dev=dev)
         return Xout
 
     def _monotone_tables(self, comps, start_distance=10, resolution=1001):
@@ -1383,9 +1459,11 @@ class transport_map():
     def evaluate_pullback_density(self, X, X_star=None):
         """tm.py:2646-2712."""
         assert self.monotonicity == "separable monotonicity", "evaluate_pushforward_density is currently only implemented for monotonicity = 'separable monotonicity'."
-        X = np.asarray(X, dtype=np.float64)
-        if X_star is not None:
-            X = np.column_stack((X_star, X))
+        X = self._samples(X, ncol=self._Dtot if X_star is None else None)
+        dev = isinstance(X, _DevSamples)
+        X = self._stack(X_star, X)
+        if dev and X.n == 0:
+            return self._empty(0)
         if self._fused_small():
             return self._map_fused(X, 0, sigma=[float(self.X_std[k]) for k in range(self.D)])[1]   # X_std[k], tm.py:2706
         n = X.shape[0]
@@ -1404,28 +1482,53 @@ class transport_map():
         out = self._empty(n)
         B.check(self._lib.ttm_density_finish(self._ctx, B.c_void_p(acc.data_ptr()), None,
                                              B.c_void_p(out.data_ptr()), n, self._stream()))
-        return self._download(out)
+        return self._result(out, dev)
+
+    def _stack(self, X_star, X):
+        """[X_star | X] (np.column_stack of tm.py:2614 / :2675) in the kind of X (host array or _DevSamples); with a
+        CUDA X the column count is checked before the device copy."""
+        if X_star is None:
+            return X
+        torch = self._torch
+        if not isinstance(X, _DevSamples):
+            if isinstance(X_star, torch.Tensor) and X_star.is_cuda:
+                X_star = X_star.to(torch.float64).cpu().numpy()
+            return np.column_stack((X_star, X))
+        Xs = self._samples(X_star)
+        if Xs.ndim != 2 or Xs.shape[1] + X.d != self._Dtot:
+            raise ValueError('operands could not be broadcast together: X_star %s and X %s, the map has %d columns'
+                             % (tuple(Xs.shape), tuple(X.shape), self._Dtot))
+        xs = Xs.t if isinstance(Xs, _DevSamples) else self._upload(Xs)
+        return self._samples(torch.cat((xs.to(torch.float64), X.t.to(torch.float64)), dim=1))
 
     def evaluate_pushforward_density(self, Z, log_target_pdf, X_star=None):
-        """tm.py:2569-2644.  `log_target_pdf` is a user Python callback on host arrays."""
+        """tm.py:2569-2644.  `log_target_pdf` is a user Python callback, called with the inverse-mapped samples: a
+        host array, or a CUDA tensor when Z is one (it may then return a CUDA tensor or a host array of length n)."""
         assert self.monotonicity == "separable monotonicity", "evaluate_pushforward_density is currently only implemented for monotonicity = 'separable monotonicity'."
+        torch = self._torch
+        dev = isinstance(Z, torch.Tensor) and Z.is_cuda
         X = self.inverse_map(Z, X_star)
-        log_target = np.ascontiguousarray(log_target_pdf(X), dtype=np.float64)
-        if X_star is not None:
-            X = np.column_stack((X_star, X))
+        n = X.shape[0]
+        if dev and n == 0:
+            return self._empty(0)
+        log_target = log_target_pdf(X)
+        if isinstance(log_target, torch.Tensor) and log_target.is_cuda:
+            lt = log_target.to(self._device, torch.float64).reshape(-1).contiguous()
+        else:
+            lt = self._upload(np.ascontiguousarray(log_target, dtype=np.float64))
+        if dev and lt.numel() != n:
+            raise ValueError('log_target_pdf returned %d values for %d samples' % (lt.numel(), n))
+        X = self._stack(X_star, self._samples(X) if dev else X)
         if self._fused_small():
             return self._map_fused(X, 1, sigma=[float(self.X_std[k + self.skip_dimensions]) for k in range(self.D)],
-                                   log_target=log_target)[1]                          # X_std[k+skip], tm.py:2638
-        n = X.shape[0]
-        torch = self._torch
+                                   log_target=lt)[1]                                  # X_std[k+skip], tm.py:2638
         Xraw_t = self._to_colmajor(X)
         acc = torch.zeros(n, dtype=torch.float64, device=self._device)
         self._log_det_accumulate(acc, Xraw_t, n, None, 1, self.skip_dimensions)   # X_std[k+skip], tm.py:2638
         out = self._empty(n)
-        lt = self._upload(log_target)
         B.check(self._lib.ttm_density_finish(self._ctx, B.c_void_p(acc.data_ptr()), B.c_void_p(lt.data_ptr()),
                                              B.c_void_p(out.data_ptr()), n, self._stream()))
-        return self._download(out)
+        return self._result(out, dev)
 
     # ================================================================== measurement helpers
     def fp64_peak_tflops(self):
