@@ -79,6 +79,81 @@ __device__ __forceinline__ void stage_table(unsigned int* s_tab, int tid, int nt
         s_tab[j] = (j < TAB_ENTRIES) ? TTM_E32_TAB_LO[j] : TTM_E32_TAB_HI[j - TAB_ENTRIES];
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// exp of a product, exp(a b), for the tile kernel's hot loops, given bK = b * K (K = E / ln2) instead of a b:
+//
+//   t = fma(a, bK, MAGIC),  nf = t - MAGIC = E n + j,  u = fma(a, bK, -nf)   (|u| <= 1/2, one rounding)
+//   exp(a b) ~ 2^(j/E) 2^n * P(u),   P(u) = 1 + u (C + u (C^2 Q0 + u (C^3 Q1 + u C^4 Q2)))  = p(C u), C = ln2/E
+//
+// i.e. the same polynomial in the unscaled variable u: 7 FP64 and the final DMUL against the scaled table word, where
+// exp(y) of a formed product y = a b takes 1 + 8.  The argument carries one rounding of b K (and of K) instead of one
+// rounding of a b and the representation error of C: exp of an argument perturbed by a relative <= 2^-52, the class of
+// the fused reduction above.  Maximum relative error of the 64-entry form on |a b| <= 40: 9.8e-15 measured, bound
+// 1.5e-14 (polynomial 5.1e-15 plus 40 * 2^-52 from the argument; tests/test_exp_product_form.py).
+//
+// Exponent insertion before the DMUL, in one IMAD: the "folded" high words hi'[j] = hi[j] - (j << 14) are staged
+// behind the table, so that for c = E (n + 1021) + j (E = 64; 2^15 and j << 15 for E = 32)
+//   hi(tb[j] 2^(n + 1021)) = hi[j] + (n + 1021) 2^20 = c 2^14 + hi'[j].
+// Scaling the table word instead of the product is exact (every intermediate stays normal and finite: c is clamped to
+// [0, TOP], or proven in range), so the result equals the scaled product bit for bit.  Without the clamp c is not
+// bounded: CLAMP_NONE is only for arguments the caller has proven to lie in [-700, 700].
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int TAB_FOLDED_WORDS = 3 * TAB_ENTRIES;           // [0..E) low | [E..2E) high | [2E..3E) folded high words
+constexpr int TAB_FOLD = 20 - TTM_E32_SHIFT;                // 14 for E = 64: c 2^14 = (n + 1021) 2^20 + j 2^14
+constexpr double PK_C1 = TTM_E32_C;
+constexpr double PK_C2 = TTM_E32_C * TTM_E32_C * TTM_E32_Q0;
+constexpr double PK_C3 = TTM_E32_C * TTM_E32_C * TTM_E32_C * TTM_E32_Q1;
+constexpr double PK_C4 = TTM_E32_C * TTM_E32_C * TTM_E32_C * TTM_E32_C * TTM_E32_Q2;
+#if TTM_E32_DEG == 5
+constexpr double PK_C5 = TTM_E32_C * TTM_E32_C * TTM_E32_C * TTM_E32_C * TTM_E32_C * TTM_E32_Q3;
+#endif
+
+enum { CLAMP_NONE = 0, CLAMP_NEG = 1, CLAMP_GEN = 2 };      // argument proven in range / <= 0 / any
+
+// stage_table's layout followed by the folded high words (TAB_FOLDED_WORDS words)
+__device__ __forceinline__ void stage_table_folded(unsigned int* s_tab, int tid, int nthreads) {
+    for (int j = tid; j < TAB_FOLDED_WORDS; j += nthreads)
+        s_tab[j] = (j < TAB_ENTRIES)       ? TTM_E32_TAB_LO[j]
+                 : (j < 2 * TAB_ENTRIES)   ? TTM_E32_TAB_HI[j - TAB_ENTRIES]
+                                           : TTM_E32_TAB_HI[j - 2 * TAB_ENTRIES] - ((unsigned)(j - 2 * TAB_ENTRIES) << TAB_FOLD);
+}
+
+template <int L, int CLAMP>
+__device__ __forceinline__ void exp_prod_v(const double (&a)[L], const double (&bK)[L], double (&out)[L],
+                                           const unsigned int* __restrict__ tab) {
+    double t[L], u[L], p[L];
+    int c[L];
+#pragma unroll
+    for (int l = 0; l < L; ++l) t[l] = fma(a[l], bK[l], TTM_E32_MAGIC);
+#pragma unroll
+    for (int l = 0; l < L; ++l) {
+        const int m = __double2loint(t[l]);
+        c[l] = (CLAMP == CLAMP_NEG) ? max(m, 0) : (CLAMP == CLAMP_GEN) ? __vimin_s32_relu(m, TTM_E32_TOP) : m;
+        u[l] = fma(a[l], bK[l], -(t[l] - TTM_E32_MAGIC));
+    }
+#if TTM_E32_DEG == 5
+#pragma unroll
+    for (int l = 0; l < L; ++l) p[l] = fma(u[l], PK_C5, PK_C4);
+#pragma unroll
+    for (int l = 0; l < L; ++l) p[l] = fma(p[l], u[l], PK_C3);
+#else
+#pragma unroll
+    for (int l = 0; l < L; ++l) p[l] = fma(u[l], PK_C4, PK_C3);
+#endif
+#pragma unroll
+    for (int l = 0; l < L; ++l) p[l] = fma(p[l], u[l], PK_C2);
+#pragma unroll
+    for (int l = 0; l < L; ++l) p[l] = fma(p[l], u[l], PK_C1);
+#pragma unroll
+    for (int l = 0; l < L; ++l) p[l] = fma(p[l], u[l], 1.0);
+#pragma unroll
+    for (int l = 0; l < L; ++l) {
+        const int j = c[l] & TTM_E32_MASK;
+        const unsigned hi = (unsigned)c[l] * (1u << TAB_FOLD) + tab[2 * TAB_ENTRIES + j];
+        out[l] = p[l] * __hiloint2double((int)hi, (int)tab[j]);
+    }
+}
+
 // hi + (c >> SHIFT) * 2^20 as SHF + IMAD (the compiler's own strength reduction takes three instructions)
 __device__ __forceinline__ int insert_exponent(int hi, int c) {
     int n, out;

@@ -14,9 +14,10 @@
 //                                  r(t) is evaluated in Horner form in the NODE variable tau = 1 + xi_q (coefficients
 //                                  rescaled per sample) and the integrals are accumulated as monomial moments in tau
 //                                  with node-only weights w tau^i; the node constants are KERNEL PARAMETERS
-//                                  (constant-bank operands indexed by the uniform loop counter), the exp table is 256
-//                                  bytes of shared memory read without bank conflicts (ttm_exp.cuh): the loop touches
-//                                  shared memory with 4 wavefronts per node and warp.  27 FP64 instructions per node.
+//                                  (constant-bank operands indexed by the uniform loop counter), the exp table is
+//                                  shared memory read without bank conflicts (ttm_exp.cuh): the loop touches
+//                                  shared memory with 4 wavefronts per node and warp.  25 FP64 instructions per node;
+//                                  warps whose exp arguments are proven in range skip the exps' clamps.
 //   phase 2  (warp <-> columns)    ONE sweep over the columns x_<c: every warp owns the dense groups g = warp (mod 8)
 //                                  and walks the tile's 8 rows of 32 samples for them: S_non partial sums per sample
 //                                  (value) and, in the same pass, h_j = sum_i w_i psi_ij (gradient) accumulated
@@ -46,7 +47,8 @@ constexpr int MAXMON = TTM_TILE_MAXMON;
 constexpr int NPARK = 8;         // L, ratio, hx*I_1..3, base_1..3
 constexpr int MAXQ = TTM_TILE_MAXQ;
 
-// node constants {tau, tau^2, w, w tau, w tau^2, w tau^3}, tau = 1 + xi_q, passed as a kernel parameter
+// node constants {tau, tau^2 K, w, w tau, w tau^2, w tau^3}, tau = 1 + xi_q, K = E / ln2 (the factor of exp_prod_v),
+// passed as a kernel parameter
 struct NodeTab {
     double v[6 * MAXQ];
 };
@@ -71,7 +73,7 @@ static_assert(sizeof(Layout) <= sizeof(((ObjArgs*)nullptr)->tile_lay), "ObjArgs:
 inline Layout make_layout(int m, int ndense, int ns, int nout, bool grad) {
     Layout L;
     int o = 0;
-    L.o_tab = o;   o += ttm_exp32::TAB_DOUBLES;       // exp table: low words | high words
+    L.o_tab = o;   o += (ttm_exp32::TAB_FOLDED_WORDS + 1) / 2;   // exp table: low | high | folded high words
     L.o_coef = o;  o += (m + 2) & ~1;
     L.o_prod = o;  o += 8 * ndense;                   // coefficient * scale, slot 2*order+hf
     L.o_col = o;   o += (ndense + 2) / 2;             // ints
@@ -158,11 +160,9 @@ __device__ __forceinline__ void sweep_tile(const double* __restrict__ Xt, int64_
             double xx[4], ga[4];
 #pragma unroll
             for (int r = 0; r < 4; ++r) xx[r] = x[r0 + r] * x[r0 + r];
-            if (SL::ANY_HF) {
-                double y[4];
-#pragma unroll
-                for (int r = 0; r < 4; ++r) y[r] = -0.25 * xx[r];
-                exp_neg_v<4>(y, ga, s_tab);
+            if (SL::ANY_HF) {                                   // e^{-x^2/4} = exp_prod(x^2, -K/4): no -x^2/4 formed
+                const double bK[4] = {-0.25 * TTM_E32_K, -0.25 * TTM_E32_K, -0.25 * TTM_E32_K, -0.25 * TTM_E32_K};
+                exp_prod_v<4, CLAMP_NEG>(xx, bK, ga, s_tab);
             }
 #pragma unroll
             for (int r = 0; r < 4; ++r) {
@@ -212,6 +212,45 @@ __device__ __forceinline__ void sweep_tile(const double* __restrict__ Xt, int64_
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// phase 1: the Gauss-Legendre node loop of one sample, NQ nodes in flight.  e^{ya tau^2} = exp_prod(ya, tau^2 K) and
+// g = exp_prod(ga, P_K(tau)) with the rectifier polynomial's coefficients EK pre-multiplied by K; Qp (a multiple of NQ)
+// nodes, constants loaded through the uniform loop counter.  The loop stays rolled: fully unrolled for Q = 100 (every
+// node constant at a fixed constant-bank address, 62 KB of code per instance) the C4 step measured 4.3 % slower, and
+// unrolled by 20 nodes 9.4 % slower (profiles/objgrad_tile_r4.json).  FAST: the caller has proven both exp arguments
+// to lie in [-700, 700] for every lane of the warp, so the exps skip their clamps (same bits in range).
+// ---------------------------------------------------------------------------------------------------------
+template <bool GRAD, int NQ, bool FAST>
+__device__ __forceinline__ void node_loop(const double* __restrict__ ntv, int Qp, double ya, const double (&EK)[4],
+                                          const unsigned int* __restrict__ s_tab, double& Sacc, double& m0, double& m1,
+                                          double& m2, double& m3) {
+#pragma unroll 1
+    for (int q = 0; q < Qp; q += NQ) {
+        double yk[NQ], yv[NQ], ga[NQ], r[NQ], g[NQ];
+        const double* nd = ntv + 6 * q;                                  // constant bank, uniform index
+#pragma unroll
+        for (int l = 0; l < NQ; ++l) { yv[l] = ya; yk[l] = nd[6 * l + 1]; }
+        exp_prod_v<NQ, FAST ? CLAMP_NONE : CLAMP_NEG>(yv, yk, ga, s_tab);
+#pragma unroll
+        for (int l = 0; l < NQ; ++l) {
+            const double tau = nd[6 * l];
+            r[l] = fma(fma(fma(EK[3], tau, EK[2]), tau, EK[1]), tau, EK[0]);
+        }
+        exp_prod_v<NQ, FAST ? CLAMP_NONE : CLAMP_GEN>(ga, r, g, s_tab);
+#pragma unroll
+        for (int l = 0; l < NQ; ++l) {
+            Sacc = fma(nd[6 * l + 2], g[l], Sacc);
+            if (GRAD) {
+                const double gg = g[l] * ga[l];
+                m0 = fma(nd[6 * l + 2], gg, m0);
+                m1 = fma(nd[6 * l + 3], gg, m1);
+                m2 = fma(nd[6 * l + 4], gg, m2);
+                m3 = fma(nd[6 * l + 5], gg, m3);
+            }
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------------------
 template <int MASK, bool GRAD, bool MERGED, int NQ>
@@ -241,7 +280,7 @@ __global__ void __launch_bounds__(TB, 2) objgrad_tile_kernel(const __grid_consta
     double* s_outv = smem + LY.o_out;
 
     // ---- stage tables
-    stage_table(s_tab, tid, TB);
+    stage_table_folded(s_tab, tid, TB);
     for (int j = tid; j < m; j += TB) s_coef[j] = a.coeffs[j];
     const int dstride = 2 * (P.dense_maxord + 1);
     for (int e = tid; e < 8 * ndense; e += TB) {
@@ -330,32 +369,14 @@ __global__ void __launch_bounds__(TB, 2) objgrad_tile_kernel(const __grid_consta
             const double hx2 = hx * hx;
             const double ya = -0.25 * hx2;
             const double E3 = C3 * (hx2 * hx), E2 = C2 * hx2, E1 = fma(-3.0, C3, C1) * hx, E0 = -C2;
+            const double EK[4] = {E0 * TTM_E32_K, E1 * TTM_E32_K, E2 * TTM_E32_K, E3 * TTM_E32_K};
             double Sacc = 0.0, m0 = 0.0, m1 = 0.0, m2 = 0.0, m3 = 0.0;   // moments of w g' e^{-t^2/4} in tau
-#pragma unroll 1
-            for (int q = 0; q < Qp; q += NQ) {
-                double y[NQ], ga[NQ], r[NQ], g[NQ];
-                const double* nd = nt.v + 6 * q;                         // constant bank, uniform index
-#pragma unroll
-                for (int l = 0; l < NQ; ++l) y[l] = ya * nd[6 * l + 1];
-                exp_neg_v<NQ>(y, ga, s_tab);
-#pragma unroll
-                for (int l = 0; l < NQ; ++l) {
-                    const double tau = nd[6 * l];
-                    r[l] = fma(fma(fma(E3, tau, E2), tau, E1), tau, E0) * ga[l];
-                }
-                exp_gen_v<NQ>(r, g, s_tab);
-#pragma unroll
-                for (int l = 0; l < NQ; ++l) {
-                    Sacc = fma(nd[6 * l + 2], g[l], Sacc);
-                    if (GRAD) {
-                        const double gg = g[l] * ga[l];
-                        m0 = fma(nd[6 * l + 2], gg, m0);
-                        m1 = fma(nd[6 * l + 3], gg, m1);
-                        m2 = fma(nd[6 * l + 4], gg, m2);
-                        m3 = fma(nd[6 * l + 5], gg, m3);
-                    }
-                }
-            }
+            // both exp arguments in [-700, 700] on every node (tau <= 2, e^{ya tau^2} <= 1; fails on NaN): no clamps
+            const double rbound = fabs(E0) + 2.0 * fabs(E1) + 4.0 * fabs(E2) + 8.0 * fabs(E3);
+            if (__all_sync(0xffffffffu, ya >= -175.0 && rbound < 700.0))
+                node_loop<GRAD, NQ, true>(nt.v, Qp, ya, EK, s_tab, Sacc, m0, m1, m2, m3);
+            else
+                node_loop<GRAD, NQ, false>(nt.v, Qp, ya, EK, s_tab, Sacc, m0, m1, m2, m3);
             // back to t = hx tau:  sum w g' e^{-t^2/4} t^i = hx^i m_i
             m1 *= hx; m2 *= hx2; m3 *= hx2 * hx;
             const double M = valid ? hx * fma(a.delta, a.wsum, Sacc) : 0.0;   // sum_q hx w_q (g_q + delta)
@@ -518,7 +539,7 @@ cudaError_t launch_mask(const ObjArgs& a_in, bool grad, int sm_count, cudaStream
         const double tau = (q < a.Q) ? 1.0 + a.h_xis[q] : 0.0, w = (q < a.Q) ? a.h_ws[q] : 0.0;
         const double t2 = tau * tau;
         double* v = nt.v + 6 * q;
-        v[0] = tau; v[1] = t2; v[2] = w; v[3] = w * tau; v[4] = w * t2; v[5] = w * (t2 * tau);
+        v[0] = tau; v[1] = t2 * TTM_E32_K; v[2] = w; v[3] = w * tau; v[4] = w * t2; v[5] = w * (t2 * tau);
     }
     const int64_t tiles = (a.N + TB - 1) / TB;
     const int bps = a.blocks_per_sm > 0 ? (a.blocks_per_sm > 2 ? 2 : a.blocks_per_sm) : 2;
