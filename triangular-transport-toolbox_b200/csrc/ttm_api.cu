@@ -663,7 +663,7 @@ int ttm_sep_objgrad(ttm_plan* p, const double* Xt, int64_t ld, int64_t N, const 
 int ttm_mon_table(ttm_plan* p, int ntab, double* table, void* stream) {
     if (!p || !table || ntab < 2) return fail(TTM_ERR_ARG, "ttm_mon_table: bad arguments");
     CK(cudaSetDevice(p->ctx->device));
-    CK(ttm_launch_mon_table(p->view, p->d_coeffs, ntab, 0, 0, table, (cudaStream_t)stream));
+    CK(ttm_launch_mon_table(p->view, p->d_coeffs, ntab, table, (cudaStream_t)stream));
     return TTM_OK;
 }
 

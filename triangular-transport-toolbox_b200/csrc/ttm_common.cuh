@@ -117,6 +117,15 @@ __device__ __forceinline__ double4 ldg_d4(const double4* p) {
     return make_double4(a.x, a.y, b.x, b.y);
 }
 
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+
+// FP64 tensor-core MMA C += A B (A 8x4, B 4x8, C 8x8): each lane holds one element of A and of B and two of C
+__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
+    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
+                 : "+d"(c0), "+d"(c1)
+                 : "d"(a), "d"(b));
+}
+
 #define TTM_INV_SQRT2 0.70710678118654752440
 #define TTM_SQRT_2PI 2.50662827463100050242
 #define TTM_SQRT_2_OVER_PI 0.79788456080286535588

@@ -21,12 +21,6 @@ constexpr int GK = 32;        // rows per staged slab
 constexpr int GLD = GT + 4;   // shared-memory row stride (doubles): conflict-free m8n8k4 fragment reads
 constexpr int T_GRAM = 256;
 
-__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
-
 // blockIdx.x = tile pair (ti <= tj, tj >= tj0), blockIdx.y = row split.  tj0 > 0: only the tile columns from tj0 on
 // (the "tail" Gram: Psi^T [last columns], all a component needs when the leading block comes from a donor).
 __global__ void __launch_bounds__(T_GRAM) syrk_dmma_kernel(const double* __restrict__ Psi, int64_t n, int Mp,

@@ -252,8 +252,7 @@ cudaError_t ttm_launch_inverse_bisect(const InvArgs& a, int sm_count, cudaStream
     return cudaGetLastError();
 }
 
-cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double, double, double* table,
-                                 cudaStream_t st) {
+cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double* table, cudaStream_t st) {
     // `table` holds the abscissae in table[ntab .. 2*ntab) on entry; values are written to table[0 .. ntab)
     mon_table_kernel<<<(ntab + 127) / 128, 128, 0, st>>>(P, coeffs, ntab, table + ntab, table);
     return cudaGetLastError();

@@ -123,8 +123,6 @@ __device__ __forceinline__ double table_lookup_smem(const double* __restrict__ t
     return __dadd_rn(__dmul_rn(__ddiv_rn(__dsub_rn(t, xl), den), yh), __dmul_rn(__ddiv_rn(__dsub_rn(xh, t), den), yl));
 }
 
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-
 // Apack: component block b holds rows v = 0 .. c0 + CB*b + CB - 1, each row CB*NS doubles [jj][slot];
 // entries with v >= c0 + CB*b + jj (not a predecessor of component jj) are zero
 __host__ __device__ inline int64_t block_row0(int b, int c0) { return (int64_t)b * (c0 + CB) + (int64_t)CB * b * (b - 1) / 2; }
@@ -357,11 +355,6 @@ constexpr int TS = 64;        // samples per tile
 constexpr int TC = 128;       // components per tile
 constexpr int FS = TS + 4;    // shared-memory row strides (doubles): conflict-free m8n8k4 fragment reads
 constexpr int AS = TC + 4;
-
-__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
 
 template <int NS>
 __global__ void __launch_bounds__(TB, 2) inverse_rect_kernel(const InvRectArgs a) {

@@ -36,7 +36,7 @@ struct ObjArgs {
     int n_out_terms;       // monotone terms with an outer product over x_<c
     const double* h_xis;   // HOST copies of the quadrature rule: the tile kernel's launcher turns them into the
     const double* h_ws;    // node-constant table it passes as a kernel parameter
-    int tile_lay[16];      // shared-memory layout of the tile kernel (offsets in doubles), computed by its launcher
+    int lay[16];           // shared-memory layout of the launched kernel (offsets in doubles), computed by its launcher
 };
 
 #define TTM_TILE_MAXMON 8   // monotone terms per component handled by the tile kernel
@@ -182,8 +182,7 @@ size_t ttm_inverse_fused_apack_doubles(int ncomp, int c0, int ns);
 
 cudaError_t ttm_launch_inverse_table(const InvArgs& a, int sm_count, cudaStream_t st);
 cudaError_t ttm_launch_inverse_bisect(const InvArgs& a, int sm_count, cudaStream_t st);
-cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double lo, double hi,
-                                 double* table, cudaStream_t st);
+cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double* table, cudaStream_t st);
 
 // FP64 pipe micro-benchmark (dependent-free DFMA chains); returns flop count per launch
 cudaError_t ttm_launch_fp64_peak(double* sink, int iters, int grid, int block, cudaStream_t st);

@@ -1,13 +1,11 @@
 // Dispatcher of K-objgrad / K-S: picks the narrowest compiled instantiation that covers the
 // component's slot structure (see ttm_objgrad_impl.cuh for the kernel).
-#include <cstdlib>
-
 #include "ttm_objgrad_impl.cuh"
 
 // Returns cudaErrorInvalidValue if the plan exceeds the compiled limits (order > 20 or > 8
 // special-term inner factors).
 cudaError_t ttm_launch_objgrad(const ObjArgs& a_in, bool grad, int sm_count, cudaStream_t st) {
-    using ttm_obj::T_OBJ;
+    using namespace ttm_obj;
     ObjArgs a = a_in;
     const PlanView& P = a.P;
     if (!grad) a.gram_mode = 0;
@@ -17,39 +15,13 @@ cudaError_t ttm_launch_objgrad(const ObjArgs& a_in, bool grad, int sm_count, cud
         if (e != cudaErrorNotSupported) return e;
     }
     if (a.gram_mode && P.dense_maxord > 3) return cudaErrorInvalidValue;   // merged sweep handles orders <= 3
-    a.ch_rows = a.gram_mode ? 2 * ttm_obj::RC_SWEEP : ttm_obj::CH_ROWS;
-    const int m = P.m_non + P.m_mon;
-    const bool herme = (P.family == FAM_HERMITE_E);
-    const bool exprect = (a.rect == RECT_EXP);
-    const int64_t rows = (a.N + T_OBJ - 1) / T_OBJ;
-    const int nslot_rt = 2 * (P.maxord + 1) + P.nst;
-    auto smem_for = [&](int maxord_t) {
-        return sizeof(double) * (size_t)(m + 2 * (a.Q + 4) + 32 + 3 * (maxord_t + 1) + nslot_rt + (grad ? (T_OBJ / 32) * (1 + m) : 0) +
-                                        (size_t)P.ndense * 2 * (P.dense_maxord + 1) * 2 + 2 * P.ndense + 6) +
-               sizeof(int) * (size_t)(P.ndense * 2 * (P.dense_maxord + 1) + 8 + nslot_rt + 2 * P.m_mon + P.n_outfac + 6) +
-               sizeof(double) * ((size_t)a.ch_rows * T_OBJ * (1 + (a.gram_mode ? 1 + P.nactive : 0)) + 2);
-    };
-    auto grid_for = [&](int blocks_per_sm) {
-        int64_t g = (int64_t)sm_count * blocks_per_sm;
-        if (g > rows) g = rows;
-        if (g > a.max_grid) g = a.max_grid;
-        return (int)(g < 1 ? 1 : g);
-    };
-    if (P.nst == 0 && herme && exprect && !P.has_plain && P.maxord <= 3) {
-        // general kernel, hot instantiation (RB = 2 samples x NQ = 2 nodes in flight per thread); reached only when the
-        // tile kernel does not cover the plan (special / multivariate nonmonotone terms, nonmonotone order > 3)
-        const int bps = a.blocks_per_sm > 0 ? a.blocks_per_sm : 4;
-        return ttm_objgrad_cfg6(a, grad, grid_for(bps), smem_for(3), st);
-    }
-    if (P.nst == 0 && herme && exprect && P.maxord <= 3)
-        return ttm_objgrad_cfg1(a, grad, grid_for(4), smem_for(3), st);
-    if (P.nst == 0 && herme && exprect && P.maxord <= 6)
-        return ttm_objgrad_cfg2(a, grad, grid_for(3), smem_for(6), st);
-    if (P.nst == 0 && herme && exprect && P.maxord <= 12)
-        return ttm_objgrad_cfg3(a, grad, grid_for(3), smem_for(12), st);
-    if (P.nst == 0 && P.maxord <= 6)
-        return ttm_objgrad_cfg4(a, grad, grid_for(3), smem_for(6), st);
-    if (P.nst <= 8 && P.maxord <= 20)
-        return ttm_objgrad_cfg5(a, grad, grid_for(2), smem_for(20), st);
+    a.ch_rows = a.gram_mode ? 2 * RC_SWEEP : CH_ROWS;
+    if (Cfg6::covers(P, a.rect)) return launch_cfg<Cfg6>(a, grad, sm_count, st);
+    a.blocks_per_sm = 0;   // the context's blocks-per-SM setting applies to the hot instantiation only
+    if (Cfg1::covers(P, a.rect)) return launch_cfg<Cfg1>(a, grad, sm_count, st);
+    if (Cfg2::covers(P, a.rect)) return launch_cfg<Cfg2>(a, grad, sm_count, st);
+    if (Cfg3::covers(P, a.rect)) return launch_cfg<Cfg3>(a, grad, sm_count, st);
+    if (Cfg4::covers(P, a.rect)) return launch_cfg<Cfg4>(a, grad, sm_count, st);
+    if (Cfg5::covers(P, a.rect)) return launch_cfg<Cfg5>(a, grad, sm_count, st);
     return cudaErrorInvalidValue;
 }

@@ -1,6 +1,4 @@
 // instantiation 1 of the K-objgrad kernel template (see ttm_objgrad_impl.cuh)
 #include "ttm_objgrad_impl.cuh"
 
-cudaError_t ttm_objgrad_cfg1(const ObjArgs& a, bool grad, int grid, size_t smem, cudaStream_t st) {
-    return ttm_obj::launch_cfg<3, true, true, 0, true, true, 2, 1>(a, grad, grid, smem, st);
-}
+template cudaError_t ttm_obj::launch_cfg<ttm_obj::Cfg1>(const ObjArgs&, bool, int, cudaStream_t);

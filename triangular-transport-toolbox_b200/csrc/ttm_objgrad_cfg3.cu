@@ -1,6 +1,4 @@
 // instantiation 3 of the K-objgrad kernel template (see ttm_objgrad_impl.cuh)
 #include "ttm_objgrad_impl.cuh"
 
-cudaError_t ttm_objgrad_cfg3(const ObjArgs& a, bool grad, int grid, size_t smem, cudaStream_t st) {
-    return ttm_obj::launch_cfg<12, true, true, 0, true, true, 1, 1>(a, grad, grid, smem, st);
-}
+template cudaError_t ttm_obj::launch_cfg<ttm_obj::Cfg3>(const ObjArgs&, bool, int, cudaStream_t);

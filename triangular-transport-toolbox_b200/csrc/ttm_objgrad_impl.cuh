@@ -48,6 +48,43 @@ __device__ __forceinline__ void ladder(double t, const double* __restrict__ rec,
     }
 }
 
+// Dynamic shared-memory layout of objgrad_kernel (offsets in doubles): the launcher sizes the launch with `total` and
+// passes the offsets in ObjArgs::lay, from which the kernel takes its pointers.
+struct Layout {
+    int o_coef, o_xis, o_ws, o_exptab, o_rec, o_scale, o_gacc;
+    int o_dense;                                      // dense-group tables (stage_dense_tables)
+    int o_slot_ptr, o_slot_term, o_out_ptr, o_out_fac;  // ints
+    int o_S, o_M, o_I, total;
+};
+static_assert(sizeof(Layout) <= sizeof(((ObjArgs*)nullptr)->lay), "ObjArgs::lay too small");
+
+// maxord, nq: the instantiation's MAXORD and NQ; gram: Gram mode (GRAD only); ch_rows: rows per chunk
+inline Layout make_layout(const PlanView& P, int Q, int maxord, int nq, bool grad, bool gram, int ch_rows) {
+    const int m = P.m_non + P.m_mon;
+    const int nslot = 2 * (P.maxord + 1) + P.nst;
+    const int qp = (Q + nq - 1) / nq * nq;            // node count padded to a multiple of NQ
+    Layout L;
+    int o = 0;
+    L.o_coef = o;      o += m;
+    L.o_xis = o;       o += qp;
+    L.o_ws = o;        o += qp;
+    L.o_exptab = o;    o += 32;                       // 2^(j/32), j < 32: the exp table of the node loop
+    L.o_rec = o;       o += 3 * (maxord + 1);         // recurrence coefficients A | B | C
+    L.o_scale = o;     o += nslot;
+    L.o_gacc = o;      o += grad ? (T_OBJ / 32) * (1 + m) : 0;   // per warp: J, gradient
+    L.o_dense = o;     o += dense_smem_doubles(P.ndense, P.dense_maxord);
+    // monotone slot tables (the per-row-group prologue/epilogue walks them; from L2 they cost ~300 cycles per hop)
+    L.o_slot_ptr = o;  o += (nslot + 2) / 2;          // [nslot + 1]
+    L.o_slot_term = o; o += (P.m_mon + 1) / 2;        // [m_mon]
+    L.o_out_ptr = o;   o += (P.m_mon + 2) / 2;        // [m_mon + 1]
+    L.o_out_fac = o;   o += (P.n_outfac + 1) / 2;     // [n_outfac]
+    L.o_S = o;         o += ch_rows * T_OBJ;          // [ch_rows][T_OBJ]
+    L.o_M = o;         o += gram ? ch_rows * T_OBJ : 0;                // [ch_rows][T_OBJ]
+    L.o_I = o;         o += gram ? P.nactive * ch_rows * T_OBJ : 0;    // [nactive][ch_rows][T_OBJ]
+    L.total = o;
+    return L;
+}
+
 // outer (x_<c) product of monotone term j on sample i; 1 if the term has no outer factor
 static __device__ __noinline__ double outer_product(const PlanView& P, const int* __restrict__ out_ptr,
                                                     const int* __restrict__ out_fac, int j,
@@ -60,7 +97,7 @@ static __device__ __noinline__ double outer_product(const PlanView& P, const int
 
 template <int MAXORD, bool HAS_PLAIN, bool HAS_HF, int NST, bool HERME, bool EXPRECT, bool GRAD, int RB, int NQ>
 __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
-    extern __shared__ double smem[];
+    extern __shared__ __align__(16) double smem[];
     const PlanView& P = a.P;
     const int m = P.m_non + P.m_mon;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -70,27 +107,22 @@ __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
     const int st_base = 2 * (P.maxord + 1);               // first special-term slot of the plan
     const int nslot_rt = st_base + P.nst;
 
-    double* s_coef = smem;
-    const int Qp = (a.Q + NQ - 1) / NQ * NQ;            // node count padded to a multiple of NQ
-    double* s_xis = s_coef + m;
-    double* s_ws = s_xis + Qp;
-    double* s_exptab = s_ws + Qp;                        // 2^(j/32), j < 32: the exp table of the node loop
-    double* s_rec = s_exptab + 32;
-    double* s_scale = s_rec + 3 * (MAXORD + 1);
-    double* s_gacc = s_scale + nslot_rt;
-    // dense nonmonotone tables staged after the gradient slots: coefficient products, scales, indices, groups
-    const int dstride = 2 * (P.dense_maxord + 1);
-    const int ndt = P.ndense * dstride;
-    double* s_dprod = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(s_gacc + (GRAD ? NW * (1 + m) : 0)) + 15) & ~uintptr_t(15));
-    double* s_dscale = s_dprod + ndt;
-    int4* s_dvar = reinterpret_cast<int4*>((reinterpret_cast<uintptr_t>(s_dscale + ndt) + 15) & ~uintptr_t(15));
-    int* s_didx = reinterpret_cast<int*>(s_dvar + P.ndense);
-    // monotone slot tables (the per-row-group prologue/epilogue walks them; from L2 they cost ~300 cycles per hop)
-    int* s_slot_ptr = s_didx + ndt;                      // [nslot_rt + 1]
-    int* s_slot_term = s_slot_ptr + nslot_rt + 1;        // [m_mon]
-    int* s_out_ptr = s_slot_term + P.m_mon;              // [m_mon + 1]
-    int* s_out_fac = s_out_ptr + P.m_mon + 1;            // [n_outfac]
-    double* s_S = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(s_out_fac + P.n_outfac) + 15) & ~uintptr_t(15));  // [ch_rows][T_OBJ]
+    const Layout& L = *reinterpret_cast<const Layout*>(a.lay);
+    const int Qp = L.o_ws - L.o_xis;                     // node count padded to a multiple of NQ
+    double* s_coef = smem + L.o_coef;
+    double* s_xis = smem + L.o_xis;
+    double* s_ws = smem + L.o_ws;
+    double* s_exptab = smem + L.o_exptab;
+    double* s_rec = smem + L.o_rec;
+    double* s_scale = smem + L.o_scale;
+    double* s_gacc = smem + L.o_gacc;
+    int* s_slot_ptr = reinterpret_cast<int*>(smem + L.o_slot_ptr);
+    int* s_slot_term = reinterpret_cast<int*>(smem + L.o_slot_term);
+    int* s_out_ptr = reinterpret_cast<int*>(smem + L.o_out_ptr);
+    int* s_out_fac = reinterpret_cast<int*>(smem + L.o_out_fac);
+    double* s_S = smem + L.o_S;
+    double* s_M = smem + L.o_M;
+    double* s_I = smem + L.o_I;
 
     for (int j = tid; j < m; j += T_OBJ) s_coef[j] = a.coeffs[j];
     for (int q = tid; q < Qp; q += T_OBJ) {              // padding nodes: mid-point, zero weight
@@ -106,24 +138,12 @@ __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
     for (int s = tid; s < nslot_rt; s += T_OBJ) s_scale[s] = P.db[P.o_d_slot_scale + s];
     if (GRAD)
         for (int j = tid; j < NW * (1 + m); j += T_OBJ) s_gacc[j] = 0.0;
-    for (int e = tid; e < ndt; e += T_OBJ) {
-        const int j = P.ib[P.o_dense_idx + e];
-        const double sc = P.db[P.o_d_dense_scale + e];
-        s_didx[e] = j;
-        s_dscale[e] = sc;
-        s_dprod[e] = (j >= 0) ? a.coeffs[j] * sc : 0.0;
-    }
-    for (int g = tid; g < P.ndense; g += T_OBJ) s_dvar[g] = reinterpret_cast<const int4*>(P.ib + P.o_dense_var)[g];
+    const DenseSmem DS = stage_dense_tables(P, a.coeffs, L.o_dense, tid, T_OBJ);
     for (int e = tid; e <= nslot_rt; e += T_OBJ) s_slot_ptr[e] = P.ib[P.o_slot_ptr + e];
     for (int e = tid; e < P.m_mon; e += T_OBJ) s_slot_term[e] = P.ib[P.o_slot_term + e];
     for (int e = tid; e <= P.m_mon; e += T_OBJ) s_out_ptr[e] = P.ib[P.o_out_ptr + e];
     for (int e = tid; e < P.n_outfac; e += T_OBJ) s_out_fac[e] = P.ib[P.o_out_fac + e];
     __syncthreads();
-    DenseTabs DT;
-    DT.var = s_dvar; DT.idx = s_didx; DT.scale = s_dscale; DT.coefprod = s_dprod;
-    DenseSmem DS;
-    DS.o_var = (int)(reinterpret_cast<double*>(s_dvar) - smem); DS.o_idx = (int)(reinterpret_cast<double*>(s_didx) - smem);
-    DS.o_scale = (int)(s_dscale - smem); DS.o_prod = (int)(s_dprod - smem);
 
     const double* acoef = s_coef;
     const double* bcoef = s_coef + P.m_non;
@@ -160,8 +180,6 @@ __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
     // Otherwise (pass 0): phase A sweep, node loop + epilogue, phase C sweep.
     const bool gm = GRAD && a.gram_mode != 0;
     const int ch_rows = a.ch_rows;
-    double* s_M = s_S + ch_rows * T_OBJ;                 // [ch_rows][T_OBJ]     (gram mode)
-    double* s_I = s_M + ch_rows * T_OBJ;                 // [nactive][ch_rows][T_OBJ]
     for (int64_t chunk_lo = row_lo; chunk_lo < row_hi; chunk_lo += ch_rows) {
     const int64_t chunk_hi = (chunk_lo + ch_rows < row_hi) ? chunk_lo + ch_rows : row_hi;
     if (!gm) {
@@ -198,8 +216,8 @@ __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
             Mv[r] = (in && pass == 2) ? s_M[(row0 + r - chunk_lo) * T_OBJ + tid] : 0.0;
         }
         // ---------------- phase A (constants, special terms, multivariate terms) ----------------
-        if (pass != 1) nonmon_sweep<false, HERME, false>(P, DT, Xt, ld, idx, acoef, S, gslot, lane);
-        if (pass == 2) nonmon_sweep<true, HERME, false>(P, DT, Xt, ld, idx, acoef, Mv, gslot, lane);  // their h_j
+        if (pass != 1) nonmon_generic_sweep<false, HERME>(P, Xt, ld, idx, acoef, S, gslot, lane);
+        if (pass == 2) nonmon_generic_sweep<true, HERME>(P, Xt, ld, idx, acoef, Mv, gslot, lane);  // their h_j
 
         // ---------------- phase B ----------------
 #pragma unroll 1
@@ -483,7 +501,7 @@ __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
         } else if (pass == 0) {
             // ---------------- phase C ----------------
             // constants / special terms / multivariate terms per row group; dense groups per chunk below
-            nonmon_sweep<true, HERME, false>(P, DT, Xt, ld, idx, acoef, S, gslot, lane);
+            nonmon_generic_sweep<true, HERME>(P, Xt, ld, idx, acoef, S, gslot, lane);
 #pragma unroll
             for (int r = 0; r < R_OBJ; ++r)
                 if (row0 + r < chunk_hi) s_S[(row0 + r - chunk_lo) * T_OBJ + tid] = S[r];
@@ -530,33 +548,53 @@ __global__ void __launch_bounds__(T_OBJ) objgrad_kernel(const ObjArgs a) {
     }
 }
 
-template <int MAXORD, bool HAS_PLAIN, bool HAS_HF, int NST, bool HERME, bool EXPRECT, int RB, int NQ>
-cudaError_t launch_cfg(const ObjArgs& a, bool grad, int grid, size_t smem, cudaStream_t st) {
-    cudaError_t e;
-    if (grad) {
-        auto k = objgrad_kernel<MAXORD, HAS_PLAIN, HAS_HF, NST, HERME, EXPRECT, true, RB, NQ>;
-        if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-        k<<<grid, T_OBJ, smem, st>>>(a);
-    } else {
-        auto k = objgrad_kernel<MAXORD, HAS_PLAIN, HAS_HF, NST, HERME, EXPRECT, false, RB, NQ>;
-        if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-        k<<<grid, T_OBJ, smem, st>>>(a);
+// One compiled instantiation: its template arguments and resident blocks per SM (BPS)
+template <int MAXORD_, bool HAS_PLAIN_, bool HAS_HF_, int NST_, bool HERME_, bool EXPRECT_, int RB_, int NQ_, int BPS_>
+struct ObjCfg {
+    static constexpr int MAXORD = MAXORD_, NST = NST_, RB = RB_, NQ = NQ_, BPS = BPS_;
+    static constexpr bool HAS_PLAIN = HAS_PLAIN_, HAS_HF = HAS_HF_, HERME = HERME_, EXPRECT = EXPRECT_;
+    // the instantiation can compute the component: within its orders and special terms, and of its family and rectifier
+    static bool covers(const PlanView& P, int rect) {
+        return P.maxord <= MAXORD && P.nst <= NST && (HAS_PLAIN || !P.has_plain) && (HAS_HF || !P.has_hf) &&
+               (!HERME || P.family == FAM_HERMITE_E) && (!EXPRECT || rect == RECT_EXP);
     }
+};
+
+//                   MAXORD  PLAIN  HF    NST  HERME  EXPRECT  RB  NQ  BPS
+using Cfg1 = ObjCfg<3,       true,  true, 0,   true,  true,    2,  1,  4>;
+using Cfg2 = ObjCfg<6,       true,  true, 0,   true,  true,    2,  1,  3>;
+using Cfg3 = ObjCfg<12,      true,  true, 0,   true,  true,    1,  1,  3>;
+using Cfg4 = ObjCfg<6,       true,  true, 0,   false, false,   2,  1,  3>;
+using Cfg5 = ObjCfg<20,      true,  true, 8,   false, false,   1,  1,  2>;
+// hot instantiation (RB = 2 samples x NQ = 2 nodes in flight per thread); reached only when the tile kernel does not
+// cover the plan (special / multivariate nonmonotone terms, nonmonotone order > 3)
+using Cfg6 = ObjCfg<3,       false, true, 0,   true,  true,    2,  2,  4>;
+
+template <class C>
+cudaError_t launch_cfg(const ObjArgs& a, bool grad, int sm_count, cudaStream_t st) {
+    const int64_t rows = (a.N + T_OBJ - 1) / T_OBJ;
+    int64_t grid = (int64_t)sm_count * (a.blocks_per_sm > 0 ? a.blocks_per_sm : C::BPS);
+    if (grid > rows) grid = rows;
+    if (grid > a.max_grid) grid = a.max_grid;
+    if (grid < 1) grid = 1;
+    ObjArgs b = a;
+    const Layout L = make_layout(a.P, a.Q, C::MAXORD, C::NQ, grad, a.gram_mode != 0, a.ch_rows);
+    *reinterpret_cast<Layout*>(b.lay) = L;
+    const size_t smem = sizeof(double) * (size_t)L.total;
+    auto k = grad ? objgrad_kernel<C::MAXORD, C::HAS_PLAIN, C::HAS_HF, C::NST, C::HERME, C::EXPRECT, true, C::RB, C::NQ>
+                  : objgrad_kernel<C::MAXORD, C::HAS_PLAIN, C::HAS_HF, C::NST, C::HERME, C::EXPRECT, false, C::RB, C::NQ>;
+    cudaError_t e;
+    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    k<<<(int)grid, T_OBJ, smem, st>>>(b);
     return cudaGetLastError();
 }
 
+// each instantiation is compiled by its own translation unit, ttm_objgrad_cfg<N>.cu
+extern template cudaError_t launch_cfg<Cfg1>(const ObjArgs&, bool, int, cudaStream_t);
+extern template cudaError_t launch_cfg<Cfg2>(const ObjArgs&, bool, int, cudaStream_t);
+extern template cudaError_t launch_cfg<Cfg3>(const ObjArgs&, bool, int, cudaStream_t);
+extern template cudaError_t launch_cfg<Cfg4>(const ObjArgs&, bool, int, cudaStream_t);
+extern template cudaError_t launch_cfg<Cfg5>(const ObjArgs&, bool, int, cudaStream_t);
+extern template cudaError_t launch_cfg<Cfg6>(const ObjArgs&, bool, int, cudaStream_t);
+
 }  // namespace ttm_obj
-
-// one exported launcher per instantiation (defined in ttm_objgrad_cfg<N>.cu)
-#define TTM_OBJ_CFG_LIST(X)                          \
-    X(1, 3, true, true, 0, true, true, 2, 1)         \
-    X(2, 6, true, true, 0, true, true, 2, 1)         \
-    X(3, 12, true, true, 0, true, true, 1, 1)        \
-    X(4, 6, true, true, 0, false, false, 2, 1)       \
-    X(5, 20, true, true, 8, false, false, 1, 1)      \
-    X(6, 3, false, true, 0, true, true, 2, 2)
-
-#define TTM_OBJ_DECL(ID, MAXORD, HP, HH, NST, HERME, EXPR, RB, NQ) \
-    cudaError_t ttm_objgrad_cfg##ID(const ObjArgs& a, bool grad, int grid, size_t smem, cudaStream_t st);
-TTM_OBJ_CFG_LIST(TTM_OBJ_DECL)
-#undef TTM_OBJ_DECL

@@ -63,12 +63,12 @@ static __device__ __noinline__ double tile_outer_product(const PlanView& P, int 
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// shared-memory layout (offsets in doubles), computed by the launcher and passed in ObjArgs::tile_lay
+// shared-memory layout (offsets in doubles), computed by the launcher and passed in ObjArgs::lay
 // ---------------------------------------------------------------------------------------------------------
 struct Layout {
     int o_tab, o_coef, o_prod, o_col, o_mon, o_M, o_park, o_u, o_Spart, o_hacc, o_red, o_out, total;
 };
-static_assert(sizeof(Layout) <= sizeof(((ObjArgs*)nullptr)->tile_lay), "ObjArgs::tile_lay too small");
+static_assert(sizeof(Layout) <= sizeof(((ObjArgs*)nullptr)->lay), "ObjArgs::lay too small");
 
 inline Layout make_layout(int m, int ndense, int ns, int nout, bool grad) {
     Layout L;
@@ -263,7 +263,7 @@ __global__ void __launch_bounds__(TB, 2) objgrad_tile_kernel(const __grid_consta
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int Qp = (a.Q + NQ - 1) / NQ * NQ;
     const int ndense = P.ndense;
-    const Layout& LY = *reinterpret_cast<const Layout*>(a.tile_lay);
+    const Layout& LY = *reinterpret_cast<const Layout*>(a.lay);
     unsigned int* s_tab = reinterpret_cast<unsigned int*>(smem + LY.o_tab);
     double* s_coef = smem + LY.o_coef;
     double* s_prod = smem + LY.o_prod;
@@ -533,7 +533,7 @@ cudaError_t launch_mask(const ObjArgs& a_in, bool grad, int sm_count, cudaStream
     const size_t smem = sizeof(double) * (size_t)LY.total;
     const int Qp = (a.Q + NQ - 1) / NQ * NQ;
     if (smem > 227 * 1024 || Qp > MAXQ || !a.h_xis || !a.h_ws) return cudaErrorInvalidValue;
-    *reinterpret_cast<Layout*>(a.tile_lay) = LY;
+    *reinterpret_cast<Layout*>(a.lay) = LY;
     NodeTab nt;
     for (int q = 0; q < Qp; ++q) {                            // padding nodes: tau = 0, zero weight
         const double tau = (q < a.Q) ? 1.0 + a.h_xis[q] : 0.0, w = (q < a.Q) ? a.h_ws[q] : 0.0;
