@@ -146,6 +146,19 @@ int ttm_density_accumulate(ttm_ctx* ctx, double* acc, const double* S, const dou
 int ttm_density_finish(ttm_ctx* ctx, const double* acc, const double* log_target, double* out, int64_t N,
                        void* stream);
 
+/* ---- K-logdet-IR ------------------------------------------------------------------------------
+ * replaces: nothing -- the reference's density evaluators assert separable monotonicity (tm.py:2569, :2646).  The
+ * log-determinant term of an integrated-rectifier component for evaluate_log_pullback_density /
+ * evaluate_log_pushforward_density: l_i = log d_c S_k(x_i) = log(g(r_i) + delta), r_i = sum_j b_j psi^mon_j(x_i)
+ * (l_i = r_i for the exponential rectifier with delta = 0), the same per-sample quantity as the objective's -log
+ * term.  Xt: standardised samples (column-major, all columns <= c); S: K-S output (ttm_eval_s_ir), read in mode 0 only.
+ *   mode 0 (pullback):    acc[i] += -S_i^2/2 - log(2 pi)/2 + l_i - log(sigma)
+ *   mode 1 (pushforward): acc[i] -= l_i - log(sigma)
+ * Coefficients as last set with ttm_plan_set_coeffs.  One thread per sample, no atomics (bit-reproducible).
+ * TTM_ERR_LIMIT for polynomial order > 32 or > 16 special inner terms (as ttm_inverse_bisect). */
+int ttm_ir_logdet_accumulate(ttm_plan* plan, const double* Xt, int64_t ld, int64_t N, const double* S, double sigma,
+                             int mode, double* acc, void* stream);
+
 /* K-map-fused / K-pullback: all D components of a (small) separable map on row-major samples in ONE launch.
  * replaces: map tm.py:2391-2437 + the whole of evaluate_pullback_density :2646-2712 / the log-determinant loop of
  * evaluate_pushforward_density :2618-2644 (the per-component entry points above remain for large maps).
@@ -154,7 +167,11 @@ int ttm_density_finish(ttm_ctx* ctx, const double* acc, const double* log_target
  * X: device row-major (n, Dtot) UNstandardised samples; mean/std: device [Dtot] or both NULL.
  *   mode 0: out[i] = pullback density, Z (optional, row-major (n, D)) = map output
  *   mode 1: out[i] = exp(log_target[i] - sum_k log(d_k S_k / sigma_k))
- *   mode 2: Z = map output only */
+ *   mode 2: Z = map output only
+ *   mode 3: out[i] = log pullback density of the fitted map (Z optional as in mode 0)
+ *   mode 4: out[i] = log_target[i] - sum_k log(d_k S_k / sigma_k)
+ * Modes 3 and 4 evaluate d_k S_k on the STANDARDISED samples and return the log (no exp); host_sigma[k] =
+ * X_std[k+skip] there (evaluate_log_pullback_density / evaluate_log_pushforward_density). */
 int ttm_map_fused(ttm_ctx* ctx, ttm_plan* const* host_plans, int D, const double* host_sigma, const double* X, int64_t n,
                   int Dtot, const double* mean, const double* std, const double* log_target, int mode, double* Z,
                   double* out, void* stream);

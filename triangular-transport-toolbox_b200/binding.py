@@ -91,6 +91,8 @@ def lib():
                                    ctypes.POINTER(c_int), c_void_p],
             'ttm_density_accumulate': [c_void_p, c_void_p, c_void_p, c_void_p, c_double, c_int, c_int64, c_void_p],
             'ttm_density_finish': [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p],
+            'ttm_ir_logdet_accumulate': [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_double, c_int, c_void_p,
+                                         c_void_p],
             'ttm_fp64_peak': [c_void_p, _dp],
         }
         for name, args in sig.items():

@@ -473,6 +473,19 @@ int ttm_density_accumulate(ttm_ctx* c, double* acc, const double* S, const doubl
     return TTM_OK;
 }
 
+int ttm_ir_logdet_accumulate(ttm_plan* p, const double* Xt, int64_t ld, int64_t N, const double* S, double sigma,
+                             int mode, double* acc, void* stream) {
+    if (!p || !Xt || !acc || N <= 0 || ld < N || mode < 0 || mode > 1 || (mode == 0 && !S) || !(sigma > 0.0))
+        return fail(TTM_ERR_ARG, "ttm_ir_logdet_accumulate: bad arguments");
+    ttm_ctx* c = p->ctx;
+    CK(cudaSetDevice(c->device));
+    cudaError_t e = ttm_launch_ir_logdet(p->view, p->d_coeffs, Xt, ld, N, S, sigma, c->rect, c->delta, mode, acc,
+                                         (cudaStream_t)stream);
+    if (e == cudaErrorInvalidValue) return fail(TTM_ERR_LIMIT, "ttm_ir_logdet_accumulate: polynomial order > 32 or > 16 special inner terms");
+    CK(e);
+    return TTM_OK;
+}
+
 int ttm_density_finish(ttm_ctx* c, const double* acc, const double* log_target, double* out, int64_t N, void* stream) {
     if (!c || !acc || !out || N <= 0) return fail(TTM_ERR_ARG, "ttm_density_finish: bad arguments");
     CK(cudaSetDevice(c->device));
@@ -483,7 +496,7 @@ int ttm_density_finish(ttm_ctx* c, const double* acc, const double* log_target, 
 int ttm_map_fused_ld(ttm_ctx* c, ttm_plan* const* host_plans, int D, const double* host_sigma, const void* X, int dtype,
                      int64_t ldx, int64_t n, int Dtot, const double* mean, const double* sd, const double* log_target,
                      int mode, double* Z, double* out, void* stream) {
-    if (!c || !host_plans || D <= 0 || !X || n <= 0 || Dtot <= 0 || mode < 0 || mode > 2 || (mode != 2 && (!out || !host_sigma)) ||
+    if (!c || !host_plans || D <= 0 || !X || n <= 0 || Dtot <= 0 || mode < 0 || mode > 4 || (mode != 2 && (!out || !host_sigma)) ||
         (mode == 2 && !Z) || ((mean == nullptr) != (sd == nullptr)) || ldx < Dtot || !known_dtype(dtype))
         return fail(TTM_ERR_ARG, "ttm_map_fused: bad arguments");
     CK(cudaSetDevice(c->device));

@@ -1,4 +1,5 @@
 // K-inv-table / K-inv-bisect: per-sample inversion of one map component, S_k(x_<c, x_c) = z_k.
+// K-logdet-IR (end of file): log d_c S_k of an integrated-rectifier component for the log-density evaluators.
 //
 // Reference: inverse_map transport_map.py:3639-3796 (host loop over k, sequential);
 //            vectorized_root_search_alternate :3987-4084 (1001-point table + scipy interp1d linear);
@@ -221,6 +222,31 @@ __global__ void mon_table_kernel(const PlanView P, const double* __restrict__ co
     table[q] = acc;
 }
 
+// K-logdet-IR: l = log d_c S_k = log(g(r(x_c)) + delta) per sample, r(t) = sum_j b_j psi^mon_j(x_<c, t) -- the
+// quantity the objective's -log term uses (ttm_objgrad_impl.cuh) -- accumulated into the log density:
+//   mode 0 (pullback):    acc += -S^2/2 - log(2 pi)/2 + l - log sigma
+//   mode 1 (pushforward): acc -= l - log sigma
+// exponential with delta = 0 gives l = r exactly (rect_log); every other case log(g + delta), the integrand of the
+// quadrature in K-S.  One thread per sample, no atomics: the result does not depend on the launch shape.
+__global__ void __launch_bounds__(T_INV) ir_logdet_kernel(const PlanView P, const double* __restrict__ coeffs,
+                                                          const double* __restrict__ Xt, int64_t ld, int64_t N,
+                                                          const double* __restrict__ S, double log_sigma, int rect,
+                                                          double delta, int mode, double* __restrict__ acc) {
+    extern __shared__ double s_b[];
+    for (int j = threadIdx.x; j < P.m_mon; j += T_INV) s_b[j] = coeffs[P.m_non + j];
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * T_INV + threadIdx.x;
+    if (i >= N) return;
+    MonEval ev;
+    ev.P = &P; ev.a = nullptr; ev.xis = nullptr; ev.ws = nullptr;
+    ev.prepare(s_b, Xt, ld, i);
+    const double r = ev.lin(Xt[(int64_t)P.c * ld + i]);
+    const double l = (rect == RECT_EXP && delta == 0.0) ? r : log(rect_eval(rect, r) + delta);
+    const double t = l - log_sigma;
+    if (mode == 0) acc[i] += -0.5 * S[i] * S[i] - 0.91893853320467274178 + t;
+    else acc[i] -= t;
+}
+
 }  // namespace
 
 cudaError_t ttm_launch_inverse_table(const InvArgs& a, int sm_count, cudaStream_t st) {
@@ -255,5 +281,20 @@ cudaError_t ttm_launch_inverse_bisect(const InvArgs& a, int sm_count, cudaStream
 cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double* table, cudaStream_t st) {
     // `table` holds the abscissae in table[ntab .. 2*ntab) on entry; values are written to table[0 .. ntab)
     mon_table_kernel<<<(ntab + 127) / 128, 128, 0, st>>>(P, coeffs, ntab, table + ntab, table);
+    return cudaGetLastError();
+}
+
+cudaError_t ttm_launch_ir_logdet(const PlanView& P, const double* coeffs, const double* Xt, int64_t ld, int64_t N,
+                                 const double* S, double sigma, int rect, double delta, int mode, double* acc,
+                                 cudaStream_t st) {
+    if (N == 0) return cudaSuccess;
+    if (2 * (P.maxord + 1) + P.nst > MAX_SLOTS) return cudaErrorInvalidValue;
+    const size_t smem = sizeof(double) * (size_t)(P.m_mon > 0 ? P.m_mon : 1);
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(ir_logdet_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    ir_logdet_kernel<<<(unsigned)((N + T_INV - 1) / T_INV), T_INV, smem, st>>>(P, coeffs, Xt, ld, N, S, log(sigma),
+                                                                              rect, delta, mode, acc);
     return cudaGetLastError();
 }

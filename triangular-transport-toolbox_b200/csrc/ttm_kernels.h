@@ -89,7 +89,8 @@ struct FusedMapArgs {
     const double* mean;      // device [Dtot] or NULL (no standardisation)
     const double* sd;
     const double* logt;      // device [n] or NULL (mode 1)
-    int mode;                // 0 pullback density (+ Z if given), 1 pushforward density, 2 map only
+    int mode;                // 0 pullback density (+ Z if given), 1 pushforward density, 2 map only,
+                             // 3 / 4 log pullback / log pushforward density (derivative basis on the standardised samples)
     double* Z;               // device row-major (n, D) or NULL
     double* out;             // device [n] (modes 0, 1)
 };
@@ -183,6 +184,10 @@ size_t ttm_inverse_fused_apack_doubles(int ncomp, int c0, int ns);
 cudaError_t ttm_launch_inverse_table(const InvArgs& a, int sm_count, cudaStream_t st);
 cudaError_t ttm_launch_inverse_bisect(const InvArgs& a, int sm_count, cudaStream_t st);
 cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double* table, cudaStream_t st);
+// K-logdet-IR (ttm_inverse.cu); cudaErrorInvalidValue if the plan has more slots than MonEval holds
+cudaError_t ttm_launch_ir_logdet(const PlanView& P, const double* coeffs, const double* Xt, int64_t ld, int64_t N,
+                                 const double* S, double sigma, int rect, double delta, int mode, double* acc,
+                                 cudaStream_t st);
 
 // FP64 pipe micro-benchmark (dependent-free DFMA chains); returns flop count per launch
 cudaError_t ttm_launch_fp64_peak(double* sink, int iters, int grid, int block, cudaStream_t st);

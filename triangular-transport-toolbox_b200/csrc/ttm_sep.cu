@@ -257,6 +257,8 @@ cudaError_t ttm_launch_sepobj_batch(const SepBatchItem* d_items, const SepBatchL
 //   pullback density    tm.py:2646-2712:  exp( sum_k [-S_k^2/2 - log(2 pi)/2] + sum_k log(dS_k / sigma_k) )
 //   pushforward density tm.py:2618-2644:  exp( log_target - sum_k log(dS_k / sigma_k) )
 // dS_k = der_Psi_mon . coeffs_mon is evaluated on the UNstandardised samples like the reference does (:2627, :2695).
+//   modes 3 / 4: the log pullback / log pushforward density of the fitted map (no exp; dS_k on the standardised
+//   samples, sigma_k = X_std[k+skip] from the host) -- evaluate_log_pullback_density / _pushforward_density.
 // HBM traffic: 8 n Dtot in, 8 n (D | 1) out.  The per-term work goes through the generic factor evaluator, so the
 // host uses this kernel for maps with a few hundred terms in total (Example 05 / 06 shapes) and the per-component
 // kernels with their dense sweeps for the large ones.
@@ -283,12 +285,14 @@ __global__ void __launch_bounds__(T_FUSE) map_fused_kernel(const FusedMapArgs a)
     }
     __syncthreads();
     if (tid >= rows) return;
+    const bool pull = a.mode == 0 || a.mode == 3, push = a.mode == 1 || a.mode == 4, logm = a.mode >= 3;
+    const double* t_der = logm ? t_std : t_raw;   // the log modes differentiate the map they evaluate
     double acc = 0.0;
     for (int k = 0; k < a.D; ++k) {
         const PlanView P = a.comps[k].P;
         const double* coef = a.comps[k].coeffs;
         const double* bcoef = coef + P.m_non;
-        if (a.mode != 1) {
+        if (!push) {
             double S = 0.0;
             for (int j = 0; j < P.m_non; ++j) S = fma(coef[j], plan_term(P, P.o_non_ptr, P.o_non_fac, j, t_std, ldt, tid), S);
             for (int j = 0; j < P.m_mon; ++j) S = fma(bcoef[j], plan_term(P, P.o_mon_ptr, P.o_mon_fac, j, t_std, ldt, tid), S);
@@ -297,12 +301,15 @@ __global__ void __launch_bounds__(T_FUSE) map_fused_kernel(const FusedMapArgs a)
         }
         if (a.mode != 2) {
             double dS = 0.0;
-            for (int j = 0; j < P.m_dmon; ++j) dS = fma(bcoef[j], plan_term(P, P.o_dmon_ptr, P.o_dmon_fac, j, t_raw, ldt, tid), dS);
+            for (int j = 0; j < P.m_dmon; ++j) dS = fma(bcoef[j], plan_term(P, P.o_dmon_ptr, P.o_dmon_fac, j, t_der, ldt, tid), dS);
             const double ld = log(dS / a.comps[k].sigma);
-            acc += (a.mode == 0) ? ld : -ld;
+            acc += pull ? ld : -ld;
         }
     }
-    if (a.mode != 2) a.out[base + tid] = exp(acc + ((a.mode == 1 && a.logt) ? a.logt[base + tid] : 0.0));
+    if (a.mode != 2) {
+        const double v = acc + ((push && a.logt) ? a.logt[base + tid] : 0.0);
+        a.out[base + tid] = logm ? v : exp(v);
+    }
 }
 
 }  // namespace

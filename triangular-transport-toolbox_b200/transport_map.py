@@ -5,7 +5,8 @@ hand-written sm_100a CUDA kernels behind the C ABI of libttm.so (include/ttm.h).
 Mirrors the reference class (`/root/reference/transport_map.py`, "tm.py"): constructor signature and
 defaults tm.py:12-39, public attributes, `optimize`, `map`, `inverse_map`, `reset`, `s`,
 `objective_function`, `objective_function_jacobian`, `evaluate_pullback_density`,
-`evaluate_pushforward_density`.  What stays on the host is what the reference's callers own: the
+`evaluate_pushforward_density`; beyond the reference, `evaluate_log_pullback_density` and
+`evaluate_log_pushforward_density` (log densities of the fitted map, both monotonicity modes).  What stays on the host is what the reference's callers own: the
 scipy optimizer steps (BFGS / L-BFGS-B, tm.py:3252-3257 / :3108-3114), the m x m linear algebra of
 the separable fit, quantile look-ups for special-term placement, and option/error handling.
 
@@ -1529,6 +1530,107 @@ class transport_map():
         B.check(self._lib.ttm_density_finish(self._ctx, B.c_void_p(acc.data_ptr()), B.c_void_p(lt.data_ptr()),
                                              B.c_void_p(out.data_ptr()), n, self._stream()))
         return self._result(out, dev)
+
+    # ================================================================== log densities (both monotonicity modes)
+    def _log_sigma(self):
+        """sigma_c = X_std[skip + k] per component (1 without standardisation)."""
+        if not self.standardize_samples:
+            return [1.0] * self.D
+        return [float(self.X_std[k + self.skip_dimensions]) for k in range(self.D)]
+
+    def _check_x_star(self, X_star, n):
+        """X_star of the log-density evaluators: the conditioning columns of a partial map, (n, skip_dimensions)."""
+        skip = self.skip_dimensions
+        if X_star is None:
+            return
+        shape = tuple(X_star.shape) if hasattr(X_star, 'shape') else np.shape(X_star)
+        if skip == 0 or len(shape) != 2 or shape[1] != skip or shape[0] != n:
+            raise ValueError('X_star must have shape (%d, skip_dimensions = %d), got %s' % (n, skip, shape))
+
+    def _log_det_terms(self, acc, Xt, n, mode):
+        """acc += sum_k [-S_k^2/2 - log(2 pi)/2 + l_k - log sigma_c] (mode 0) or acc -= sum_k [l_k - log sigma_c]
+        (mode 1) on the standardised column-major samples Xt, l_k = log d_c S_k."""
+        ir = self.monotonicity == "integrated rectifier"
+        S = self._empty(n) if mode == 0 else None
+        dS = None if ir else self._empty(n)
+        ptr = lambda t: B.c_void_p(t.data_ptr()) if t is not None else None
+        st = self._stream()
+        for k, sigma in enumerate(self._log_sigma()):
+            self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
+            if S is not None:
+                self._s_device(k, Xt, n, S)
+            if ir:
+                B.check(self._lib.ttm_ir_logdet_accumulate(self._plans[k], ptr(Xt), Xt.shape[1], n, ptr(S), sigma,
+                                                           mode, ptr(acc), st))
+            else:
+                B.check(self._lib.ttm_sep_eval(self._plans[k], None, 0, n, None, ptr(Xt), Xt.shape[1], ptr(dS), st))
+                B.check(self._lib.ttm_density_accumulate(self._ctx, ptr(acc), ptr(S), ptr(dS), sigma, mode, n, st))
+
+    def _standardized_colmajor(self, X):
+        if self.standardize_samples:
+            return self._to_colmajor(X, self._mean_d, self._std_d)
+        return self._to_colmajor(X)
+
+    def evaluate_log_pullback_density(self, X, X_star=None):
+        """log rho(x) = sum_k [-S_k(x~)^2/2 - log(2 pi)/2 + l_k(x~) - log sigma_c], the log density the fitted map pulls
+        back from the standard Gaussian, for both monotonicity modes (DESIGN.md section 1).
+
+        x are samples in the caller's units; x~ = (x - X_mean) / X_std with standardize_samples, else x~ = x and
+        sigma = 1 (the X passed is used).  c = skip_dimensions + k, sigma_c = X_std[c], and l_k = log dS_k/dx~_c:
+        integrated rectifier log(g(r_k(x~)) + delta), r_k = sum_j b_j psi^mon_j at the upper limit x~_c (r_k itself for
+        the exponential rectifier with delta = 0); separable log(der_Psi_mon(x~) . b).  On the training ensemble
+        -mean log rho = sum_k J_k + D/2 log(2 pi) + sum_k log sigma_c, J_k the objective optimize() minimises.
+        With X_star ((n, skip_dimensions), partial maps only) the result is the conditional log density of X given
+        X_star; X then has D columns, otherwise skip_dimensions + D.  X / X_star: host arrays or CUDA tensors; the
+        result (n,) float64 follows X.  Unlike evaluate_pullback_density it returns the log (no underflow in high
+        dimension) and differentiates the map it evaluates."""
+        X = self._samples(X, ncol=self._Dtot if X_star is None else self.D)
+        dev = isinstance(X, _DevSamples)
+        if X.ndim != 2 or X.shape[1] != (self._Dtot if X_star is None else self.D):
+            raise ValueError('X has shape %s; the map expects %d columns' %
+                             (tuple(X.shape), self._Dtot if X_star is None else self.D))
+        n = X.shape[0]
+        self._check_x_star(X_star, n)
+        if n == 0:
+            return self._empty(0) if dev else np.empty(0)
+        X = self._stack(X_star, X)
+        if self._fused_small():
+            return self._map_fused(X, 3, sigma=self._log_sigma())[1]
+        Xt = self._standardized_colmajor(X)
+        acc = self._torch.zeros(n, dtype=self._torch.float64, device=self._device)
+        self._log_det_terms(acc, Xt, n, 0)
+        return self._result(acc, dev)
+
+    def evaluate_log_pushforward_density(self, Z, log_target_pdf, X_star=None):
+        """log p(z) = log_target_pdf(x) - sum_k [l_k(x~) - log sigma_c], x = inverse_map(Z, X_star): the log density of
+        the samples the map pushes forward from `log_target_pdf`, for both monotonicity modes (l_k, sigma_c and X_star
+        as in evaluate_log_pullback_density).  `log_target_pdf` is called with the inverse-mapped samples (n, D) in the
+        caller's units: a host array, or a CUDA tensor when Z is one; it returns n values (host array or CUDA
+        tensor).  The result (n,) float64 follows Z."""
+        torch = self._torch
+        Z = self._samples(Z, ncol=self.D)
+        dev = isinstance(Z, _DevSamples)
+        if Z.ndim != 2 or Z.shape[1] != self.D:
+            raise ValueError('Z has shape %s; the map has %d components' % (tuple(Z.shape), self.D))
+        n = Z.shape[0]
+        self._check_x_star(X_star, n)
+        if n == 0:
+            return self._empty(0) if dev else np.empty(0)
+        X = self.inverse_map(Z, X_star)
+        log_target = log_target_pdf(X)
+        if isinstance(log_target, torch.Tensor) and log_target.is_cuda:
+            lt = log_target.to(self._device, torch.float64).reshape(-1).contiguous()
+        else:
+            lt = self._upload(np.ascontiguousarray(log_target, dtype=np.float64).reshape(-1))
+        if lt.numel() != n:
+            raise ValueError('log_target_pdf returned %d values for %d samples' % (lt.numel(), n))
+        X = self._stack(X_star, self._samples(X) if dev else X)
+        if self._fused_small():
+            return self._map_fused(X, 4, sigma=self._log_sigma(), log_target=lt)[1]
+        Xt = self._standardized_colmajor(X)
+        acc = lt.clone()
+        self._log_det_terms(acc, Xt, n, 1)
+        return self._result(acc, dev)
 
     # ================================================================== measurement helpers
     def fp64_peak_tflops(self):
