@@ -34,7 +34,12 @@ typedef struct ttm_plan ttm_plan; /* one compiled map component (term tables + w
 #define TTM_OK 0
 #define TTM_ERR_CUDA -1
 #define TTM_ERR_ARG -2
-#define TTM_ERR_LIMIT -3 /* plan exceeds a compiled limit (order > 20, > 8 special inner terms) */
+#define TTM_ERR_LIMIT -3 /* plan exceeds a compiled limit (order > 20, > 8 special inner terms), or a table is longer
+                          * than TTM_INVERSE_FUSED_MAX_NTAB (ttm_inverse_fused, ttm_inverse_fused_split) */
+
+/* longest table ttm_inverse_fused and ttm_inverse_fused_split accept: each block stages two [values | abscissae]
+ * tables (4 ntab doubles = 64 KB at the limit) in shared memory next to its coefficient operands */
+#define TTM_INVERSE_FUSED_MAX_NTAB 2048
 
 /* element type of a caller's row-major sample array (the *_ld entry points); float32 is widened on load */
 #define TTM_DTYPE_F64 0
@@ -243,7 +248,7 @@ int ttm_inverse_table(ttm_plan* plan, double* Xt, int64_t ld, int64_t N, const d
  * the constant terms' coefficients.  Apack (ttm_inverse_fused_apack_size doubles) holds coefficient*scale in blocks
  * of 16 components: block b = rows v = 0 .. c0 + 16 b + 15, row = [16 components][ns slots], zero where variable v is
  * not a predecessor of the component; ns = 3: slots {He1, He2 e^{-x^2/4}, He3 e^{-x^2/4}}, ns = 6: {He1, He1 e, He2,
- * He2 e, He3, He3 e}. */
+ * He2 e, He3, He3 e}.  ntab > TTM_INVERSE_FUSED_MAX_NTAB fails with TTM_ERR_LIMIT before any launch. */
 int ttm_inverse_fused_apack_size(int ncomp, int c0, int ns, int64_t* host_doubles);
 int ttm_inverse_fused(ttm_ctx* ctx, double* Xw, int64_t ld, int64_t N, const double* Zt, int64_t ldz, int ncomp, int c0,
                       int ns, const double* Apack, const double* a0, const double* tables, int ntab, int truncate,
@@ -253,7 +258,8 @@ int ttm_inverse_fused(ttm_ctx* ctx, double* Xw, int64_t ld, int64_t N, const dou
  * base[j][i] = sum_{v<c0} sum_q f_q(x_iv) Rpack[j/128][v][q][j%128] (features formed once per sample and variable
  * instead of once per block of 16 components), then K-inv-fused starts from `base` and walks only the columns it
  * solves.  Rpack (ttm_inverse_rect_rpack_size doubles) = [ceil(ncomp/128)][c0 rounded up to 8][ns][128], zero padded;
- * base = device scratch [ncomp][ldb], 16-byte aligned, ldb even and >= N. */
+ * base = device scratch [ncomp][ldb], 16-byte aligned, ldb even and >= N.  ntab > TTM_INVERSE_FUSED_MAX_NTAB fails
+ * with TTM_ERR_LIMIT before either launch. */
 int ttm_inverse_rect_rpack_size(int ncomp, int c0, int ns, int64_t* host_doubles);
 int ttm_inverse_fused_split(ttm_ctx* ctx, double* Xw, int64_t ld, int64_t N, const double* Zt, int64_t ldz, int ncomp,
                             int c0, int ns, const double* Apack, const double* Rpack, const double* a0,

@@ -264,6 +264,45 @@ def test_split_inverse_matches_the_oracle(D, E, n, mixed, monkeypatch):
     assert rel_err(tm.inverse_map(Z.copy(), xs()), got) <= 1e-12
 
 
+def test_fused_inverse_rejects_tables_longer_than_the_limit():
+    """ttm_inverse_fused and ttm_inverse_fused_split stage two tables per block in shared memory: ntab = 2049 (one past
+    TTM_INVERSE_FUSED_MAX_NTAB) fails with TTM_ERR_LIMIT before any launch and leaves the output untouched; ntab = 2048
+    runs and solves the column (zero offsets, identity table, z = 0 -> x = 0 up to rounding)."""
+    import torch
+    from cases import c5_terms
+    from ttt_b200 import binding as B
+    mon, non = c5_terms(2)
+    tm = make_cuda(synthetic_samples(200, 2, seed=1), monotone=mon, nonmonotone=non,
+                   monotonicity='separable monotonicity')
+    lib, n, ns = tm._lib, 8, 3
+    f64 = dict(dtype=torch.float64, device=tm._device)
+    size = B.c_int64()
+    B.check(lib.ttm_inverse_fused_apack_size(1, 1, ns, B.ctypes.byref(size)))
+    A = torch.zeros(size.value, **f64)
+    B.check(lib.ttm_inverse_rect_rpack_size(1, 1, ns, B.ctypes.byref(size)))
+    R = torch.zeros(size.value, **f64)
+    a0, Zt, base = torch.zeros(1, **f64), torch.zeros(1, n, **f64), torch.zeros(1, n, **f64)
+    p = lambda t: B.c_void_p(t.data_ptr())
+    for ntab, rc_want in ((2049, -3), (2048, 0)):
+        grid = torch.linspace(-10, 10, ntab, **f64)
+        tabs = torch.cat((grid, grid))
+        for split in (False, True):
+            Xw = torch.full((2, n), 7.0, **f64)
+            if split:
+                rc = lib.ttm_inverse_fused_split(tm._ctx, p(Xw), n, n, p(Zt), n, 1, 1, ns, p(A), p(R), p(a0), p(tabs), ntab,
+                                                 0, p(base), n, tm._stream())
+            else:
+                rc = lib.ttm_inverse_fused(tm._ctx, p(Xw), n, n, p(Zt), n, 1, 1, ns, p(A), p(a0), p(tabs), ntab, 0,
+                                           tm._stream())
+            assert rc == rc_want, (ntab, split, lib.ttm_last_error())
+            torch.cuda.synchronize(tm._device)
+            if rc_want:
+                assert b'TTM_INVERSE_FUSED_MAX_NTAB' in lib.ttm_last_error()
+                assert torch.equal(Xw, torch.full_like(Xw, 7.0))
+            else:
+                assert torch.equal(Xw[0], torch.full_like(Xw[0], 7.0)) and float(Xw[1].abs().max()) <= 1e-12
+
+
 @pytest.mark.parametrize('D,n,mixed', [(40, 4100, False), (34, 4097, True), (150, 4160, False)])
 def test_gemm_forward_map_matches_the_oracle(D, n, mixed, monkeypatch):
     """map() of a wide separable map: nonmonotone sums of all components as one block-triangular DMMA GEMM

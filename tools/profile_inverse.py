@@ -22,9 +22,10 @@ zt, t_h2d = T(lambda: tm._to_colmajor(Z))
 xs, t_h2d2 = T(lambda: tm._to_colmajor(Xstar, tm._mean_d[:E].contiguous(), tm._std_d[:E].contiguous()))
 Xw = torch.zeros(D, ns, dtype=torch.float64, device='cuda'); Xw[:E] = xs
 def comps():
-    for i, k in enumerate(range(E, D)):
-        tm._set_coeffs(k, tm.coeffs_nonmon[k], tm.coeffs_mon[k])
-        tm._root_search_table(k, Xw, ns, zt[i])
+    os.environ['TTM_INV_FUSED'] = '0'            # the per-component K-inv-table path
+    tm._inverse_solve(tm._inverse_solver([(i, k) for i, k in enumerate(range(E, D))], True), Xw, ns, ns, zt, ns,
+                      tm._stream())
+    del os.environ['TTM_INV_FUSED']
 _, t_comp = T(comps)
 _, t_d2h = T(lambda: tm._to_rowmajor(Xw, ns, D, tm._mean_d, tm._std_d))
 print(json.dumps({'total_s': t_all, 'h2d_Z_s': t_h2d, 'h2d_Xstar_s': t_h2d2, 'components_s': t_comp, 'd2h_s': t_d2h}))

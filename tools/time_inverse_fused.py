@@ -73,10 +73,10 @@ Xw2[:E] = Xw[:E, :m]
 Zt2 = Zt[:, :m].contiguous()
 torch.cuda.synchronize()
 t0 = time.perf_counter()
-for i, k in comps:
-    tm._set_coeffs(k, tm.coeffs_nonmon[k], tm.coeffs_mon[k])
-    tm._root_search_table(k, Xw2, m, Zt2[i])
+os.environ['TTM_INV_FUSED'] = '0'
+tm._inverse_solve(tm._inverse_solver(comps, True), Xw2, m, m, Zt2, m, tm._stream())
 torch.cuda.synchronize()
+del os.environ['TTM_INV_FUSED']
 out['per_component_s_200k'] = time.perf_counter() - t0
 out['max_abs_diff_vs_per_component'] = float((Xf[:, :m] - Xw2[E:]).abs().max())
 print(json.dumps(out))

@@ -711,11 +711,15 @@ int ttm_inverse_fused_apack_size(int ncomp, int c0, int ns, int64_t* host_double
     return TTM_OK;
 }
 
+static const std::string fused_ntab_limit =
+    "ntab exceeds TTM_INVERSE_FUSED_MAX_NTAB = " + std::to_string(TTM_INVERSE_FUSED_MAX_NTAB) + " (tables are staged in shared memory)";
+
 int ttm_inverse_fused(ttm_ctx* c, double* Xw, int64_t ld, int64_t N, const double* Zt, int64_t ldz, int ncomp, int c0, int ns,
                       const double* Apack, const double* a0, const double* tables, int ntab, int truncate, void* stream) {
     if (!c || !Xw || !Zt || !Apack || !a0 || !tables || N <= 0 || ld < N || ldz < N || ncomp <= 0 || c0 < 0 || ntab < 2)
         return fail(TTM_ERR_ARG, "ttm_inverse_fused: bad arguments");
     if (ns != 3 && ns != 6) return fail(TTM_ERR_ARG, "ttm_inverse_fused: ns must be 3 or 6");
+    if (ntab > TTM_INVERSE_FUSED_MAX_NTAB) return fail(TTM_ERR_LIMIT, "ttm_inverse_fused: " + fused_ntab_limit);
     CK(cudaSetDevice(c->device));
     InvFusedArgs a;
     a.Xw = Xw; a.ld = ld; a.N = N; a.Zt = Zt; a.ldz = ldz; a.ncomp = ncomp; a.c0 = c0; a.ns = ns;
@@ -738,6 +742,7 @@ int ttm_inverse_fused_split(ttm_ctx* c, double* Xw, int64_t ld, int64_t N, const
         ncomp <= 0 || c0 <= 0 || ntab < 2)
         return fail(TTM_ERR_ARG, "ttm_inverse_fused_split: bad arguments");
     if (ns != 3 && ns != 6) return fail(TTM_ERR_ARG, "ttm_inverse_fused_split: ns must be 3 or 6");
+    if (ntab > TTM_INVERSE_FUSED_MAX_NTAB) return fail(TTM_ERR_LIMIT, "ttm_inverse_fused_split: " + fused_ntab_limit);
     if ((ldb & 1) || (reinterpret_cast<uintptr_t>(base) & 15))
         return fail(TTM_ERR_ARG, "ttm_inverse_fused_split: base must be 16-byte aligned with an even leading dimension");
     CK(cudaSetDevice(c->device));

@@ -119,6 +119,28 @@ __device__ __forceinline__ double4 ldg_d4(const double4* p) {
 
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
+// Table root finder of vectorized_root_search_alternate (transport_map.py:4047-4076) for one target t: tab =
+// [sorted values | abscissae in the same order], ntab entries each.  truncate clamps t to the values' range (:4074-4076),
+// then numpy.searchsorted(side='left'), clip(1, ntab - 1) and scipy's interp1d._call_linear formula, every operation
+// correctly rounded as numpy does it.  Callers pass their shared-memory copy of the table.
+__device__ __forceinline__ double interp_sorted_table(const double* __restrict__ tab, int ntab, int truncate,
+                                                      double t) {
+    if (truncate) {
+        const double tmin = tab[0], tmax = tab[ntab - 1];
+        if (t < tmin) t = tmin;
+        if (t > tmax) t = tmax;
+    }
+    int lo = 0, hi = ntab;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (tab[mid] < t) lo = mid + 1; else hi = mid;
+    }
+    const int k = lo < 1 ? 1 : (lo > ntab - 1 ? ntab - 1 : lo);
+    const double xl = tab[k - 1], xh = tab[k], yl = tab[ntab + k - 1], yh = tab[ntab + k];
+    const double den = __dsub_rn(xh, xl);
+    return __dadd_rn(__dmul_rn(__ddiv_rn(__dsub_rn(t, xl), den), yh), __dmul_rn(__ddiv_rn(__dsub_rn(xh, t), den), yl));
+}
+
 // FP64 tensor-core MMA C += A B (A 8x4, B 4x8, C 8x8): each lane holds one element of A and of B and two of C
 __device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
     asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"

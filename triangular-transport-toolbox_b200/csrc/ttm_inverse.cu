@@ -76,65 +76,53 @@ struct MonEval {
     }
 };
 
+// Prologue shared by K-inv-table and K-inv-bisect, which both handle the samples [a.first, a.first + a.count), grid
+// striding over groups of R_OBJ rows of T_INV samples.  Dynamic shared memory holds the coefficients, the kernel's own
+// arrays, then the dense-group tables DS (each kernel stages them itself: with the staging in a helper, ptxas spills
+// more in K-inv-bisect).  Here: the thread's R_OBJ samples of row group row0 (rows past the range read sample a.first
+// and are not ok) and their nonmonotone offsets (:4039-4043).
+__device__ __forceinline__ void inv_offsets(const InvArgs& a, const DenseSmem& DS, int64_t row0, int64_t (&idx)[R_OBJ],
+                                            bool (&ok)[R_OBJ], double (&S)[R_OBJ]) {
+    const int64_t rows = (a.count + T_INV - 1) / T_INV;
+#pragma unroll
+    for (int r = 0; r < R_OBJ; ++r) {
+        const int64_t i = a.first + (row0 + r) * T_INV + threadIdx.x;
+        ok[r] = (row0 + r < rows) && (i < a.first + a.count);
+        idx[r] = ok[r] ? i : a.first;
+        S[r] = 0.0;
+    }
+    dense_value_smem_rt<R_OBJ>(a.P, DS, a.Xt, a.ld, a.first + row0 * T_INV + threadIdx.x, T_INV, ok, S);
+    nonmon_slow_rt<false>(a.P, a.Xt, a.ld, idx, ttm_dyn_smem, S, nullptr, 0);
+}
+
 __global__ void __launch_bounds__(T_INV) inverse_table_kernel(const InvArgs a) {
-    extern __shared__ double sm[];
     const PlanView& P = a.P;
     const int m = P.m_non + P.m_mon;
-    double* s_coef = sm;
-    double* s_out = s_coef + m;          // sorted table values
-    double* s_pts = s_out + a.ntab;      // abscissae
-    for (int j = threadIdx.x; j < m; j += T_INV) s_coef[j] = a.coeffs[j];
-    for (int j = threadIdx.x; j < 2 * a.ntab; j += T_INV) s_out[j] = a.table[j];
+    double* s_table = ttm_dyn_smem + m;  // [sorted values | abscissae]
+    for (int j = threadIdx.x; j < m; j += T_INV) ttm_dyn_smem[j] = a.coeffs[j];
+    for (int j = threadIdx.x; j < 2 * a.ntab; j += T_INV) s_table[j] = a.table[j];
     const DenseSmem DS = stage_dense_tables(P, a.coeffs, m + 2 * a.ntab, threadIdx.x, T_INV);
     __syncthreads();
-    const double tmin = s_out[0], tmax = s_out[a.ntab - 1];
-    const int64_t rows = (a.N + T_INV - 1) / T_INV;
+    const int64_t rows = (a.count + T_INV - 1) / T_INV;
     double* xc_col = a.Xt + (int64_t)P.c * a.ld;
     for (int64_t row0 = (int64_t)blockIdx.x * R_OBJ; row0 < rows; row0 += (int64_t)gridDim.x * R_OBJ) {
         int64_t idx[R_OBJ];
         bool ok[R_OBJ];
         double S[R_OBJ];
+        inv_offsets(a, DS, row0, idx, ok, S);
 #pragma unroll
-        for (int r = 0; r < R_OBJ; ++r) {
-            const int64_t i = (row0 + r) * T_INV + threadIdx.x;
-            ok[r] = (row0 + r < rows) && (i < a.N);
-            idx[r] = ok[r] ? i : a.N - 1;
-            S[r] = 0.0;
-        }
-        dense_value_smem_rt<R_OBJ>(P, DS, a.Xt, a.ld, row0 * T_INV + threadIdx.x, T_INV, ok, S);   // offset (:4039-4043)
-        nonmon_slow_rt<false>(P, a.Xt, a.ld, idx, s_coef, S, nullptr, 0);
-#pragma unroll
-        for (int r = 0; r < R_OBJ; ++r) {
-            if (!ok[r]) continue;
-            double t = __dadd_rn(-S[r], a.z[idx[r]]);                        // target = -offset + Zk (:4071)
-            if (a.truncate) {                                                // :4074-4076
-                if (t < tmin) t = tmin;
-                if (t > tmax) t = tmax;
-            }
-            // numpy.searchsorted(side='left') then clip(1, n-1)   (scipy interp1d._call_linear)
-            int lo = 0, hi = a.ntab;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (s_out[mid] < t) lo = mid + 1; else hi = mid;
-            }
-            int k = lo < 1 ? 1 : (lo > a.ntab - 1 ? a.ntab - 1 : lo);
-            const double xl = s_out[k - 1], xh = s_out[k], yl = s_pts[k - 1], yh = s_pts[k];
-            const double den = __dsub_rn(xh, xl);
-            const double v = __dadd_rn(__dmul_rn(__ddiv_rn(__dsub_rn(t, xl), den), yh),
-                                       __dmul_rn(__ddiv_rn(__dsub_rn(xh, t), den), yl));
-            xc_col[idx[r]] = v;
-        }
+        for (int r = 0; r < R_OBJ; ++r)
+            if (ok[r])   // target = -offset + Zk (:4071)
+                xc_col[idx[r]] = interp_sorted_table(s_table, a.ntab, a.truncate, __dadd_rn(-S[r], a.z[idx[r]]));
     }
 }
 
 __global__ void __launch_bounds__(T_INV) inverse_bisect_kernel(const InvArgs a) {
-    extern __shared__ double sm[];
     const PlanView& P = a.P;
     const int m = P.m_non + P.m_mon;
-    double* s_coef = sm;
-    double* s_xis = s_coef + m;
+    double* s_xis = ttm_dyn_smem + m;
     double* s_ws = s_xis + a.Q;
-    for (int j = threadIdx.x; j < m; j += T_INV) s_coef[j] = a.coeffs[j];
+    for (int j = threadIdx.x; j < m; j += T_INV) ttm_dyn_smem[j] = a.coeffs[j];
     for (int q = threadIdx.x; q < a.Q; q += T_INV) {
         s_xis[q] = a.xis[q];
         s_ws[q] = a.ws[q];
@@ -150,15 +138,7 @@ __global__ void __launch_bounds__(T_INV) inverse_bisect_kernel(const InvArgs a) 
         int64_t idx[R_OBJ];
         bool ok[R_OBJ];
         double S[R_OBJ];
-#pragma unroll
-        for (int r = 0; r < R_OBJ; ++r) {
-            const int64_t i = a.first + (row0 + r) * T_INV + threadIdx.x;
-            ok[r] = (row0 + r < rows) && (i < a.first + a.count);
-            idx[r] = ok[r] ? i : a.first;
-            S[r] = 0.0;
-        }
-        dense_value_smem_rt<R_OBJ>(P, DS, a.Xt, a.ld, a.first + row0 * T_INV + threadIdx.x, T_INV, ok, S);
-        nonmon_slow_rt<false>(P, a.Xt, a.ld, idx, s_coef, S, nullptr, 0);
+        inv_offsets(a, DS, row0, idx, ok, S);
 #pragma unroll 1
         for (int r = 0; r < R_OBJ; ++r) {
             if (!ok[r]) continue;
@@ -166,7 +146,7 @@ __global__ void __launch_bounds__(T_INV) inverse_bisect_kernel(const InvArgs a) 
             if (isnan(xc_col[i])) continue;                                  // marked for removal (:3846)
             MonEval ev;
             ev.P = &P; ev.a = &a; ev.xis = s_xis; ev.ws = s_ws;
-            ev.prepare(s_coef + P.m_non, a.Xt, a.ld, i);
+            ev.prepare(ttm_dyn_smem + P.m_non, a.Xt, a.ld, i);
             const double off = S[r], z = a.z[i];
             auto resid = [&](double x) { return (off + ev.mon(x)) - z; };
             double lo = -2.0, hi = 2.0;                                      // start_distance (:3850-3864)
@@ -249,33 +229,29 @@ __global__ void __launch_bounds__(T_INV) ir_logdet_kernel(const PlanView P, cons
 
 }  // namespace
 
-cudaError_t ttm_launch_inverse_table(const InvArgs& a, int sm_count, cudaStream_t st) {
-    if (a.N == 0) return cudaSuccess;
-    const int64_t rows = (a.N + T_INV - 1) / T_INV;
-    int64_t grid = (rows + R_OBJ - 1) / R_OBJ;
-    if (grid > (int64_t)sm_count * 16) grid = (int64_t)sm_count * 16;
-    const size_t smem = sizeof(double) * (size_t)(a.P.m_non + a.P.m_mon + 2 * a.ntab + dense_smem_doubles(a.P.ndense, a.P.dense_maxord));
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(inverse_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-    }
-    inverse_table_kernel<<<(unsigned)grid, T_INV, smem, st>>>(a);
-    return cudaGetLastError();
-}
-
-cudaError_t ttm_launch_inverse_bisect(const InvArgs& a, int sm_count, cudaStream_t st) {
+// K-inv-table / K-inv-bisect: at most 16 blocks per SM, each striding over groups of R_OBJ rows of T_INV samples;
+// shared memory: coefficients, the kernel's `own` doubles, dense-group tables
+static cudaError_t inv_launch(void (*kernel)(InvArgs), const InvArgs& a, int own, int sm_count, cudaStream_t st) {
     if (a.count == 0) return cudaSuccess;
-    if (2 * (a.P.maxord + 1) + a.P.nst > MAX_SLOTS) return cudaErrorInvalidValue;
     const int64_t rows = (a.count + T_INV - 1) / T_INV;
     int64_t grid = (rows + R_OBJ - 1) / R_OBJ;
     if (grid > (int64_t)sm_count * 16) grid = (int64_t)sm_count * 16;
-    const size_t smem = sizeof(double) * (size_t)(a.P.m_non + a.P.m_mon + 2 * a.Q + dense_smem_doubles(a.P.ndense, a.P.dense_maxord));
+    const size_t smem = sizeof(double) * (size_t)(a.P.m_non + a.P.m_mon + own + dense_smem_doubles(a.P.ndense, a.P.dense_maxord));
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(inverse_bisect_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    inverse_bisect_kernel<<<(unsigned)grid, T_INV, smem, st>>>(a);
+    kernel<<<(unsigned)grid, T_INV, smem, st>>>(a);
     return cudaGetLastError();
+}
+
+cudaError_t ttm_launch_inverse_table(const InvArgs& a, int sm_count, cudaStream_t st) {
+    return inv_launch(inverse_table_kernel, a, 2 * a.ntab, sm_count, st);
+}
+
+cudaError_t ttm_launch_inverse_bisect(const InvArgs& a, int sm_count, cudaStream_t st) {
+    if (a.count > 0 && 2 * (a.P.maxord + 1) + a.P.nst > MAX_SLOTS) return cudaErrorInvalidValue;
+    return inv_launch(inverse_bisect_kernel, a, 2 * a.Q, sm_count, st);
 }
 
 cudaError_t ttm_launch_mon_table(const PlanView& P, const double* coeffs, int ntab, double* table, cudaStream_t st) {

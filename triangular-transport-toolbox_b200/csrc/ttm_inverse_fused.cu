@@ -57,92 +57,26 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N)); }
 
-// numpy.searchsorted(side='left') + clip + scipy interp1d._call_linear, exactly as inverse_table_kernel
-__device__ __forceinline__ double table_lookup(const double* __restrict__ tab, int ntab, int truncate, double t) {
-    const double tmin = __ldg(tab), tmax = __ldg(tab + ntab - 1);
-    if (truncate) {
-        if (t < tmin) t = tmin;
-        if (t > tmax) t = tmax;
-    }
-    int lo = 0, hi = ntab;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (__ldg(tab + mid) < t) lo = mid + 1; else hi = mid;
-    }
-    const int k = lo < 1 ? 1 : (lo > ntab - 1 ? ntab - 1 : lo);
-    const double xl = __ldg(tab + k - 1), xh = __ldg(tab + k), yl = __ldg(tab + ntab + k - 1), yh = __ldg(tab + ntab + k);
-    const double den = __dsub_rn(xh, xl);
-    return __dadd_rn(__dmul_rn(__ddiv_rn(__dsub_rn(t, xl), den), yh), __dmul_rn(__ddiv_rn(__dsub_rn(xh, t), den), yl));
-}
-
-// The same look-up with the first levels of the binary search served from shared memory: `coarse` holds every
-// `stride`-th table value (nco <= 32 entries), the remaining <= stride entries are searched in global memory, where
-// they span two or three cache lines.  Returns exactly what table_lookup returns (searchsorted is a property of the
-// sorted array, not of the search order); cuts the dependent L2 round trips per look-up from ~10 to ~2.
-__device__ __forceinline__ double table_lookup_2level(const double* __restrict__ tab, const double* __restrict__ coarse,
-                                                      int ntab, int stride, int nco, double tmax, int truncate, double t) {
-    if (truncate) {
-        const double tmin = coarse[0];
-        if (t < tmin) t = tmin;
-        if (t > tmax) t = tmax;
-    }
-    int lo = 0, hi = nco;
-    while (lo < hi) {                                   // first coarse entry >= t
-        const int mid = (lo + hi) >> 1;
-        if (coarse[mid] < t) lo = mid + 1; else hi = mid;
-    }
-    const int ci = lo;
-    if (ci == 0) { lo = 0; hi = 0; }
-    else { lo = stride * (ci - 1) + 1; hi = (ci == nco) ? ntab : stride * ci; }
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (__ldg(tab + mid) < t) lo = mid + 1; else hi = mid;
-    }
-    const int k = lo < 1 ? 1 : (lo > ntab - 1 ? ntab - 1 : lo);
-    const double xl = __ldg(tab + k - 1), xh = __ldg(tab + k), yl = __ldg(tab + ntab + k - 1), yh = __ldg(tab + ntab + k);
-    const double den = __dsub_rn(xh, xl);
-    return __dadd_rn(__dmul_rn(__ddiv_rn(__dsub_rn(t, xl), den), yh), __dmul_rn(__ddiv_rn(__dsub_rn(xh, t), den), yl));
-}
-
-// The same look-up in a table staged in shared memory ([values | abscissae], 2 ntab doubles): ten dependent LDS instead of
-// dependent L2 round trips -- ncu attributed 37 % of the walk's issue slots to long-scoreboard waits of the search.
-__device__ __forceinline__ double table_lookup_smem(const double* __restrict__ tab, int ntab, int truncate, double t) {
-    if (truncate) {
-        const double tmin = tab[0], tmax = tab[ntab - 1];
-        if (t < tmin) t = tmin;
-        if (t > tmax) t = tmax;
-    }
-    int lo = 0, hi = ntab;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (tab[mid] < t) lo = mid + 1; else hi = mid;
-    }
-    const int k = lo < 1 ? 1 : (lo > ntab - 1 ? ntab - 1 : lo);
-    const double xl = tab[k - 1], xh = tab[k], yl = tab[ntab + k - 1], yh = tab[ntab + k];
-    const double den = __dsub_rn(xh, xl);
-    return __dadd_rn(__dmul_rn(__ddiv_rn(__dsub_rn(t, xl), den), yh), __dmul_rn(__ddiv_rn(__dsub_rn(xh, t), den), yl));
-}
-
 // Apack: component block b holds rows v = 0 .. c0 + CB*b + CB - 1, each row CB*NS doubles [jj][slot];
 // entries with v >= c0 + CB*b + jj (not a predecessor of component jj) are zero
 __host__ __device__ inline int64_t block_row0(int b, int c0) { return (int64_t)b * (c0 + CB) + (int64_t)CB * b * (b - 1) / 2; }
 
-// STAGE = 1: the component's table travels through shared memory (cp.async, double buffered, one barrier per component)
-// and the binary search runs there; 0 (tables too long for shared memory): the two-level search reads them in place.
-// (A four-level search over a bank-skewed table image -- 21 independent comparisons instead of 10 dependent halvings --
-// was measured 2 % SLOWER: the walk is bound by the dependent FP64 chains of the whole component step, not by the search.)
-template <int NS, int STAGE>
+// The component's table travels through shared memory (cp.async, double buffered, one barrier per component) and the
+// binary search runs there: ten dependent LDS instead of dependent L2 round trips -- ncu attributed 37 % of the walk's
+// issue slots to long-scoreboard waits of the search in place.  The entry points reject tables longer than
+// TTM_INVERSE_FUSED_MAX_NTAB, whose two buffers would not fit next to the operands.  (A four-level search over a
+// bank-skewed table image -- 21 independent comparisons instead of 10 dependent halvings -- was measured 2 % SLOWER: the
+// walk is bound by the dependent FP64 chains of the whole component step, not by the search.)
+template <int NS>
 __global__ void __launch_bounds__(TB, 3) inverse_fused_kernel(const InvFusedArgs a) {
     extern __shared__ double smem[];
     constexpr int ROW = CB * NS;                 // doubles per coefficient row
     unsigned int* s_tab = reinterpret_cast<unsigned int*>(smem);   // exp table (64 words)
     double* s_coef = smem + ttm_exp32::TAB_DOUBLES;   // [2][VC][ROW]
     double* s_diag = s_coef + 2 * VC * ROW;      // [CB][ROW]
-    double* s_coarse = s_diag + CB * ROW;        // [CB][33]: every stride-th table value of the block's components | tmax
-    double* s_table = s_coarse + CB * 33;        // STAGE: [2][2 ntab]
+    double* s_table = s_diag + CB * ROW;         // [2][2 ntab]
     const int tbuf = 2 * a.ntab;
     const int tid = threadIdx.x;
-    const int stride = (a.ntab + 31) / 32, nco = (a.ntab + stride - 1) / stride;
     constexpr int PF = 8;                        // variables ahead of use for the L2 prefetch of the sample columns
     ttm_exp32::stage_table(s_tab, tid, TB);
     __syncthreads();
@@ -192,16 +126,8 @@ __global__ void __launch_bounds__(TB, 3) inverse_fused_kernel(const InvFusedArgs
                     for (int e = tid; e < a.ntab; e += TB) cp_async16(dst + 2 * e, src + 2 * e);
                 }
             };
-            if (STAGE) stage_table(0);                            // buffer 0 was last read two barriers ago
+            stage_table(0);                                       // buffer 0 was last read two barriers ago
             cp_async_commit();
-            if (!STAGE)
-            for (int e = tid; e < CB * 33; e += TB) {             // coarse tables of the block (visible after the next barrier)
-                const int jj = e / 33, c = e - jj * 33, j = CB * b + jj;
-                if (j < a.ncomp) {
-                    const double* tab = a.tables + (int64_t)j * 2 * a.ntab;
-                    s_coarse[e] = (c == 32) ? __ldg(tab + a.ntab - 1) : ((c < nco) ? __ldg(tab + c * stride) : 0.0);
-                }
-            }
             {                                                     // reference samples of the block -> L2
                 const int j0 = CB * b, j1 = min(a.ncomp, j0 + CB);
                 for (int j = j0; j < j1; ++j)
@@ -282,16 +208,15 @@ __global__ void __launch_bounds__(TB, 3) inverse_fused_kernel(const InvFusedArgs
 #pragma unroll
             for (int jj = 0; jj < CB; ++jj) {
                 const int j = CB * b + jj;
-                if (STAGE && jj > 0) {                            // (jj = 0 landed with the diagonal rows)
+                if (jj > 0) {                                     // (jj = 0 landed with the diagonal rows)
                     cp_async_wait<0>();
                     __syncthreads();                              // table jj visible; everyone is done with table jj - 1
                 }
-                if (STAGE && jj + 1 < CB) {
+                if (jj + 1 < CB) {
                     stage_table(jj + 1);
                     cp_async_commit();
                 }
                 if (j < a.ncomp) {
-                    const double* tab = a.tables + (int64_t)j * 2 * a.ntab;
                     const double a0 = __ldg(a.a0 + j);
                     double xs[SPT], zc[SPT];
 #pragma unroll
@@ -304,9 +229,7 @@ __global__ void __launch_bounds__(TB, 3) inverse_fused_kernel(const InvFusedArgs
                     for (int s = 0; s < SPT; ++s) {
                         const double S = acc[s][jj] + a0;                        // offset (:4039-4043)
                         const double t = __dadd_rn(-S, zc[s]);                   // target = -offset + Zk (:4071)
-                        xs[s] = STAGE ? table_lookup_smem(s_table + (jj & 1) * tbuf, a.ntab, a.truncate, t)
-                                      : table_lookup_2level(tab, s_coarse + jj * 33, a.ntab, stride, nco,
-                                                            s_coarse[jj * 33 + 32], a.truncate, t);
+                        xs[s] = interp_sorted_table(s_table + (jj & 1) * tbuf, a.ntab, a.truncate, t);
                         if (ok[s]) a.Xw[(int64_t)(a.c0 + j) * a.ld + i[s]] = xs[s];
                     }
                     if (jj + 1 < CB && j + 1 < a.ncomp) {
@@ -499,11 +422,10 @@ size_t ttm_inverse_fused_apack_doubles(int ncomp, int c0, int ns) {
 cudaError_t ttm_launch_inverse_fused(const InvFusedArgs& a, int sm_count, cudaStream_t st) {
     using namespace ttm_invf;
     if (a.N == 0 || a.ncomp == 0) return cudaSuccess;
-    if (a.ns != 3 && a.ns != 6) return cudaErrorInvalidValue;
+    if ((a.ns != 3 && a.ns != 6) || a.ntab > TTM_INVERSE_FUSED_MAX_NTAB) return cudaErrorInvalidValue;
     const int64_t tiles = (a.N + TB * SPT - 1) / (TB * SPT);
-    const size_t smem0 = sizeof(double) * (size_t)(ttm_exp32::TAB_DOUBLES + (2 * VC + CB) * CB * a.ns + CB * 33);
-    const int stage = a.ntab <= 2048 ? 1 : 0;            // 2 x [values | abscissae] <= 64 KB next to the operands
-    const size_t smem = smem0 + sizeof(double) * (stage ? 4 * (size_t)a.ntab : 0);
+    // exp table, coefficient chunks, diagonal rows, 2 x [values | abscissae]
+    const size_t smem = sizeof(double) * (size_t)(ttm_exp32::TAB_DOUBLES + (2 * VC + CB) * CB * a.ns + 4 * a.ntab);
     cudaError_t e;
     // persistent grid = resident blocks (a block past residency would run alone on its SM at the end)
     auto launch = [&](auto kernel) -> cudaError_t {
@@ -515,6 +437,5 @@ cudaError_t ttm_launch_inverse_fused(const InvFusedArgs& a, int sm_count, cudaSt
         kernel<<<(unsigned)grid, TB, smem, st>>>(a);
         return cudaGetLastError();
     };
-    if (stage == 1) return a.ns == 3 ? launch(inverse_fused_kernel<3, 1>) : launch(inverse_fused_kernel<6, 1>);
-    return a.ns == 3 ? launch(inverse_fused_kernel<3, 0>) : launch(inverse_fused_kernel<6, 0>);
+    return a.ns == 3 ? launch(inverse_fused_kernel<3>) : launch(inverse_fused_kernel<6>);
 }

@@ -28,6 +28,10 @@ from .plan import ComponentPlan, resolve_family
 
 _RECT = {'exponential': 0, 'softplus': 1, 'squared': 2, 'expneg': 3, 'explinearunit': 4}
 
+# grid of the table root finder: the reference's start_distance = 10 and resolution = 1001 of
+# vectorized_root_search_alternate (tm.py:4047), which inverse_map never overrides
+_TABLE_HALF_WIDTH, _TABLE_NTAB = 10, 1001
+
 
 def _torch():
     import torch
@@ -1181,16 +1185,7 @@ class transport_map():
             self._to_colmajor(X_star, self._mean_d[:E].contiguous() if std else None,
                               self._std_d[:E].contiguous() if std else None, out=Xw)
         Zt = self._to_colmajor(Z)
-        fused = self._inverse_fused_setup(comps) if table_mode else None
-        if fused is not None:
-            self._inverse_fused_launch(fused, Xw, Xw.shape[1], N, Zt, Zt.shape[1])
-            comps = []
-        for i, k in comps:
-            self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
-            if table_mode:
-                self._root_search_table(k, Xw, N, Zt[i])
-            else:
-                self._root_search_bisection(k, Xw, N, Zt[i])
+        self._inverse_solve(self._inverse_solver(comps, table_mode), Xw, Xw.shape[1], N, Zt, Zt.shape[1], self._stream())
         if self.standardize_samples:
             Xout = self._to_rowmajor(Xw[skip:], N, ncol - skip, self._mean_d[skip:].contiguous(),
                                      self._std_d[skip:].contiguous(), dev=dev)
@@ -1198,18 +1193,19 @@ class transport_map():
             Xout = self._to_rowmajor(Xw[skip:], N, ncol - skip, dev=dev)
         return Xout
 
-    def _monotone_tables(self, comps, start_distance=10, resolution=1001):
+    def _monotone_tables(self, comps):
         """Lookup tables of vectorized_root_search_alternate (tm.py:4047-4062) for all listed components in ONE device
-        buffer [ncomp][2*resolution] (values | abscissae) with ONE host round trip: scipy's interp1d sorts its
+        buffer [ncomp][2*_TABLE_NTAB] (values | abscissae) with ONE host round trip: scipy's interp1d sorts its
         abscissae with a stable sort (assume_sorted=False), which is the identity for a non-decreasing table -- the
-        normal case (monotone coefficients >= 0); only rows that are not sorted are sorted on the host."""
-        pts = np.linspace(-start_distance, start_distance, resolution)
-        tabs = self._empty(len(comps), 2 * resolution)
-        tabs[:, resolution:] = self._upload(pts)
+        normal case (monotone coefficients >= 0); only rows that are not sorted are sorted on the host.  Sets the
+        components' coefficients on their plans."""
+        pts = np.linspace(-_TABLE_HALF_WIDTH, _TABLE_HALF_WIDTH, _TABLE_NTAB)
+        tabs = self._empty(len(comps), 2 * _TABLE_NTAB)
+        tabs[:, _TABLE_NTAB:] = self._upload(pts)
         for r, (_, k) in enumerate(comps):
             self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
-            B.check(self._lib.ttm_mon_table(self._plans[k], resolution, B.c_void_p(tabs[r].data_ptr()), self._stream()))
-        vals = tabs[:, :resolution].cpu().numpy()
+            B.check(self._lib.ttm_mon_table(self._plans[k], _TABLE_NTAB, B.c_void_p(tabs[r].data_ptr()), self._stream()))
+        vals = tabs[:, :_TABLE_NTAB].cpu().numpy()
         bad = np.nonzero(~np.all(vals[:, 1:] >= vals[:, :-1], axis=1))[0]
         for r in bad:
             ind = np.argsort(vals[r], kind="mergesort")
@@ -1247,7 +1243,7 @@ class transport_map():
         cache[skey] = st
         return st
 
-    def _inverse_fused_setup(self, comps, resolution=1001):
+    def _inverse_fused_setup(self, comps):
         """Operands of K-inv-fused (ttm_inverse_fused: the component loop of tm.py:3684-3698 in one launch), or None if
         some component is outside its class (nonmonotone terms other than constants and per-variable Hermite-function
         groups of order <= 3, components not on consecutive columns)."""
@@ -1262,7 +1258,7 @@ class transport_map():
             h.update(np.ascontiguousarray(self.coeffs_nonmon[k], dtype=np.float64).tobytes())
             h.update(np.ascontiguousarray(self.coeffs_mon[k], dtype=np.float64).tobytes())
         mode = os.environ.get('TTM_INV_SPLIT', 'auto')
-        key = (tuple(ks), resolution, self._ensemble_version, h.digest(), mode)
+        key = (tuple(ks), self._ensemble_version, h.digest(), mode)
         hit = getattr(self, '_inv_fused_cache', None)
         if hit is not None and hit[0] == key:
             return hit[1]
@@ -1281,7 +1277,7 @@ class transport_map():
             R = np.zeros(st['r_size'])
             R[st['rdst']] = val[st['rkeep']]
         fused = {'ncomp': ncomp, 'c0': c0, 'ns': ns, 'A': self._upload(A), 'a0': self._upload(a0),
-                 'tabs': self._monotone_tables(comps, resolution=resolution), 'ntab': resolution,
+                 'tabs': self._monotone_tables(comps), 'ntab': _TABLE_NTAB,
                  'R': self._upload(R) if split else None}
         self._inv_fused_cache = (key, fused)
         return fused
@@ -1303,27 +1299,40 @@ class transport_map():
                                             1 if self.root_search_truncation else 0,
                                             stream if stream is not None else self._stream()))
 
-    def _monotone_table(self, k, start_distance=10, resolution=1001):
-        """The lookup table of vectorized_root_search_alternate (tm.py:4047-4062) for component k (coefficients
-        already set): monotone part on a grid, evaluated on the device, sorted on the host like scipy's interp1d.
-        It depends on the coefficients only, not on the samples."""
-        pts = np.linspace(-start_distance, start_distance, resolution)
-        tab = self._empty(2 * resolution)
-        tab[resolution:] = self._upload(pts)
-        B.check(self._lib.ttm_mon_table(self._plans[k], resolution, B.c_void_p(tab.data_ptr()), self._stream()))
-        out = tab[:resolution].cpu().numpy()
-        ind = np.argsort(out, kind="mergesort")
-        return self._upload(np.concatenate((out[ind], pts[ind])))
+    def _inverse_solver(self, comps, table_mode):
+        """What _inverse_solve runs for the components `comps`: K-inv-fused with its operands, else one launch per
+        component -- K-inv-table with its row of _monotone_tables, or K-inv-bisect.  Sets the coefficients the
+        per-component launches read."""
+        fused = self._inverse_fused_setup(comps) if table_mode else None
+        if fused is not None:
+            return {'fused': fused}
+        if table_mode:
+            return {'comps': comps, 'tabs': self._monotone_tables(comps)}
+        for _, k in comps:
+            self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
+        return {'comps': comps, 'tabs': None}
 
-    def _root_search_table(self, k, Xw, N, z, start_distance=10, resolution=1001):
-        """vectorized_root_search_alternate (tm.py:3987-4084): table on the device, argsort on the host
-        (scipy interp1d sorts its abscissae), interpolation per sample on the device."""
-        tab = self._monotone_table(k, start_distance, resolution)
-        B.check(self._lib.ttm_inverse_table(self._plans[k], B.c_void_p(Xw.data_ptr()), Xw.shape[1], N,
-                                            B.c_void_p(z.data_ptr()), B.c_void_p(tab.data_ptr()), resolution,
-                                            1 if self.root_search_truncation else 0, self._stream()))
+    def _inverse_solve(self, solver, Xw, ld, n, Zt, ldz, stream, base=None):
+        """The component loop of inverse_map (tm.py:3684-3698) on n samples: solves the columns of Xw (leading dimension
+        ld) from the reference samples of component i at Zt + i*ldz.  Table mode: vectorized_root_search_alternate
+        (:3987-4084); otherwise vectorized_root_search_bisection (:3798-3985), at most 100 iterations."""
+        if 'fused' in solver:
+            self._inverse_fused_launch(solver['fused'], Xw, ld, n, Zt, ldz, stream=stream, base=base)
+            return
+        xw, trunc, tabs = B.c_void_p(Xw.data_ptr()), 1 if self.root_search_truncation else 0, solver['tabs']
+        sep = 1 if self.monotonicity.lower() == 'separable monotonicity' else 0
+        for r, (i, k) in enumerate(solver['comps']):
+            z = B.c_void_p(Zt.data_ptr() + i * ldz * 8)
+            if tabs is not None:
+                B.check(self._lib.ttm_inverse_table(self._plans[k], xw, ld, n, z, B.c_void_p(tabs[r].data_ptr()),
+                                                    _TABLE_NTAB, trunc, stream))
+                continue
+            stalled = B.c_int(0)
+            B.check(self._lib.ttm_inverse_bisect(self._plans[k], xw, ld, n, z, sep, 100, B.ctypes.byref(stalled), stream))
+            if stalled.value and self.verbose:
+                print('WARNING: root search for %d particles stopped at maximum iterations.' % stalled.value)
 
-    def _inverse_map_pipelined(self, Z, X_star, E, ncol, comps, resolution=1001):
+    def _inverse_map_pipelined(self, Z, X_star, E, ncol, comps):
         """Table-mode inverse_map for large sample counts.  Samples are independent (tm.py:3684-3698 loops over the
         components, never across samples), so the call is cut into chunks of samples that flow through four
         slots: host threads stage chunk c+1 into pinned memory (page-locked inputs are copied from directly) while
@@ -1336,12 +1345,8 @@ class transport_map():
         N, nz, skip = Z.shape[0], Z.shape[1], self.skip_dimensions
         nout = ncol - skip
         std = self.standardize_samples
-        fused = self._inverse_fused_setup(comps, resolution=resolution)
-        tabs = []
-        if fused is None:
-            for _, k in comps:                               # tables first: they need a host round trip each
-                self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
-                tabs.append(self._monotone_table(k, resolution=resolution))
+        solver = self._inverse_solver(comps, True)
+        fused = solver.get('fused')
         mean_in = self._mean_d[:E].contiguous() if (std and E > 0) else None
         std_in = self._std_d[:E].contiguous() if (std and E > 0) else None
         mean_out = self._mean_d[skip:].contiguous() if std else None
@@ -1356,7 +1361,7 @@ class transport_map():
             q = (hi - lo) // 4
             bounds = bounds[:-1] + [lo + 2 * q, lo + 3 * q, hi]
         bounds = [b for i, b in enumerate(bounds) if i == 0 or b > bounds[i - 1]]
-        nslot = min(int(os.environ.get('TTM_INV_SLOTS', 4)), len(bounds) - 1)
+        nslot = min(4, len(bounds) - 1)
         f64 = torch.float64
 
         def pinned(a):                                       # caller's array already page-locked: DMA straight from it
@@ -1380,11 +1385,10 @@ class transport_map():
                          if fused is not None and fused.get('R') is not None else None),
                 'out': torch.empty((cap, nout), dtype=f64, device=dev)})
         out_host = torch.empty((N, nout), dtype=f64, pin_memory=True)
-        trunc = 1 if self.root_search_truncation else 0
         ptr = lambda t: B.c_void_p(t.data_ptr()) if t is not None else None
         # host threads of the pageable -> pinned staging copies (memcpy-bound: ~8 GB/s per thread against 55 GB/s of PCIe)
         from .parallel import world as _world
-        nthr = int(os.environ.get('TTM_INV_STAGE_THREADS', 0)) or max(2, min(8, (os.cpu_count() or 8) // max(1, _world()[1])))
+        nthr = max(2, min(8, (os.cpu_count() or 8) // max(1, _world()[1])))
 
         def stage(dst, src, n):                              # pageable -> pinned, split over host threads
             edges = [n * t // nthr for t in range(nthr + 1)]
@@ -1416,12 +1420,7 @@ class transport_map():
                         sl['dx'][:n].copy_(src_x, non_blocking=True)
                         B.check(lib.ttm_standardize_transpose(self._ctx, ptr(sl['dx']), n, E, ptr(mean_in), ptr(std_in),
                                                               ptr(sl['Xw']), cap, st))
-                    if fused is not None:
-                        self._inverse_fused_launch(fused, sl['Xw'], cap, n, sl['Zt'], cap, stream=st, base=sl['base'])
-                    for (i, k), tab in zip(comps, tabs):
-                        B.check(lib.ttm_inverse_table(self._plans[k], ptr(sl['Xw']), cap, n,
-                                                      B.c_void_p(sl['Zt'].data_ptr() + i * cap * 8), ptr(tab),
-                                                      resolution, trunc, st))
+                    self._inverse_solve(solver, sl['Xw'], cap, n, sl['Zt'], cap, st, base=sl['base'])
                     B.check(lib.ttm_transpose_back(self._ctx, B.c_void_p(sl['Xw'].data_ptr() + skip * cap * 8), cap, n,
                                                    nout, ptr(mean_out), ptr(std_out), ptr(sl['out']), nout, st))
                     out_host[c0:c1].copy_(sl['out'][:n], non_blocking=True)
@@ -1431,16 +1430,6 @@ class transport_map():
             if sl['event'] is not None:
                 sl['event'].synchronize()
         return out_host.numpy()
-
-    def _root_search_bisection(self, k, Xw, N, z, max_iterations=100):
-        """vectorized_root_search_bisection (tm.py:3798-3985), one thread per sample."""
-        stalled = B.c_int(0)
-        sep = 1 if self.monotonicity.lower() == 'separable monotonicity' else 0
-        B.check(self._lib.ttm_inverse_bisect(self._plans[k], B.c_void_p(Xw.data_ptr()), Xw.shape[1], N,
-                                             B.c_void_p(z.data_ptr()), sep, max_iterations,
-                                             B.ctypes.byref(stalled), self._stream()))
-        if stalled.value and self.verbose:
-            print('WARNING: root search for %d particles stopped at maximum iterations.' % stalled.value)
 
     # ================================================================== densities (separable only)
     def _log_det_accumulate(self, acc, Xraw_t, n, Zt, mode, std_offset):
