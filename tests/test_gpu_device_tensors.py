@@ -109,6 +109,9 @@ def test_views_and_float32_ex06_cycle():
                           tm.inverse_map(np.ascontiguousarray(Zfull[:, 1:]), np.ascontiguousarray(X[:, :1])))
     assert np.array_equal(back(tm, tm.evaluate_pullback_density(Xd[:, 1:], X_star=Xd[:, :1])),
                           tm.evaluate_pullback_density(np.ascontiguousarray(X[:, 1:]), X_star=X[:, :1].copy()))
+    # a 1-D host X_star is one column, as np.column_stack (tm.py:2675) takes it
+    assert np.array_equal(tm.evaluate_pullback_density(np.ascontiguousarray(X[:, 1:]), X_star=X[:, 0].copy()),
+                          tm.evaluate_pullback_density(np.ascontiguousarray(X[:, 1:]), X_star=X[:, :1].copy()))
     host = tm.evaluate_pushforward_density(np.ascontiguousarray(Zfull[:, 1:]), lg, X_star=X[:, :1].copy())
     assert np.array_equal(back(tm, tm.evaluate_pushforward_density(Zd[:, 1:], lg, X_star=Xd[:, :1])), host)
     assert np.array_equal(back(tm, tm.evaluate_pushforward_density(Zd[:, 1:], lambda x: lg(x.cpu().numpy()),
@@ -251,7 +254,7 @@ def test_side_stream_results_equal_default_stream():
 
 
 # ---------------------------------------------------------------------------------------------- errors, edges
-def test_shape_errors_and_empty_inputs():
+def test_shape_errors_and_empty_inputs(monkeypatch):
     tm, X = _ex06_map()
     Dtot, D = X.shape[1], tm.D
     Xd = cuda(X)
@@ -279,6 +282,19 @@ def test_shape_errors_and_empty_inputs():
                      (tm.evaluate_pullback_density(empty[:, 1:], X_star=empty[:, :1]), (0,))):
         assert isinstance(r, torch.Tensor) and r.is_cuda and tuple(r.shape) == shape
     assert tuple(tm.inverse_map(empty[:, 1:]).shape) == (0, D)
+    lg = lambda x: -0.5 * np.sum(x ** 2, axis=1)
+    host_empty = np.zeros((0, Dtot))
+    for r in (tm.evaluate_pullback_density(host_empty),
+              tm.evaluate_pullback_density(host_empty[:, 1:], X_star=host_empty[:, :1]),
+              tm.evaluate_pushforward_density(host_empty[:, 1:], lg),
+              tm.evaluate_pushforward_density(host_empty[:, 1:], lg, X_star=host_empty[:, :1])):
+        assert isinstance(r, np.ndarray) and r.dtype == np.float64 and r.shape == (0,)
+
+    monkeypatch.setenv('TTM_MAP_FUSED', '0')              # per-component path: host arrays are checked there too
+    for bad, star in ((np.zeros((8, Dtot + 1)), None), (np.zeros((8, D)), X[:8, :2].copy()),
+                      (np.zeros((8, D)), X[:9, :1].copy())):
+        with pytest.raises(ValueError):
+            tm.evaluate_pullback_density(bad, X_star=star)
 
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs two GPUs')

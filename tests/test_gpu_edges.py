@@ -96,7 +96,7 @@ def test_order_above_compiled_limit_raises():
         tm.objective_function(np.zeros(2), 0, 1)
 
 
-def test_reset_changes_ensemble_size_and_special_terms():
+def test_reset_changes_ensemble_size_and_special_terms(monkeypatch):
     mon, non = ex05_terms()
     X1, X2 = synthetic_samples(500, 2, seed=1), synthetic_samples(1300, 2, seed=2) * 2 + 1
     kw = dict(monotone=mon, nonmonotone=non, monotonicity='separable monotonicity')
@@ -113,6 +113,13 @@ def test_reset_changes_ensemble_size_and_special_terms():
         assert rel_err(tm.coeffs_nonmon[k], om.coeffs_nonmon[k]) <= 1e-6
     Xe = synthetic_samples(77, 2, seed=3)
     assert rel_err(tm.evaluate_pullback_density(Xe.copy()), om.evaluate_pullback_density(Xe.copy())) <= 1e-9
+    # X_star on a full map (inverse_map's conditional branch): the stacked [X_star | inverse_map(Z, X_star)] has D + E
+    # columns, which only the per-component path takes (K-map-fused reads skip_dimensions + D)
+    monkeypatch.setenv('TTM_MAP_FUSED', '0')
+    Zc = np.random.default_rng(4).standard_normal((77, 1))
+    lg = lambda x: -0.5 * np.sum(x ** 2, axis=1)
+    assert rel_err(tm.evaluate_pushforward_density(Zc.copy(), lg, X_star=Xe[:, :1].copy()),
+                   om.evaluate_pushforward_density(Zc.copy(), lg, X_star=Xe[:, :1].copy())) <= 1e-9
 
 
 def test_public_attributes_and_callables_match_reference_surface():

@@ -261,8 +261,12 @@ def test_empty_and_errors():
             tm.evaluate_log_pullback_density(np.zeros((5, tm.D)), X_star=np.zeros((5, 1)))
         with pytest.raises(ValueError):
             tm.evaluate_log_pushforward_density(np.zeros((5, tm.D)), _log_gauss, X_star=np.zeros((5, 1)))
-        with pytest.raises(ValueError):                                   # callback of the wrong length
-            tm.evaluate_log_pushforward_density(np.zeros((5, tm.D)), lambda x: np.zeros(4))
+        for lt in (np.zeros(4), np.zeros(6)):                             # callback of the wrong length
+            with pytest.raises(ValueError):
+                tm.evaluate_log_pushforward_density(np.zeros((5, tm.D)), lambda x: lt)
+            if tm.monotonicity == 'separable monotonicity':               # the reference's evaluator too
+                with pytest.raises(ValueError):
+                    tm.evaluate_pushforward_density(np.zeros((5, tm.D)), lambda x: lt)
 
 
 # ---------------------------------------------------------------------------------------------- 7. full size

@@ -66,11 +66,11 @@ def c4_map(X, Q, D=64):
 
 def logdet_alone(tm, X):
     """64 K-logdet-IR launches on the standardised samples and a fixed S; coefficients set once per plan."""
-    n = X.shape[0]
-    Xt = tm._standardized_colmajor(tm._samples(X, ncol=tm._Dtot))
+    Xs, n, _ = tm._density_input(X, None, tm._Dtot)
+    Xt = tm._to_colmajor(Xs, tm._mean_d, tm._std_d)                 # the C4 map standardises its samples
     S = torch.zeros(n, dtype=torch.float64, device=X.device)
     acc = torch.zeros(n, dtype=torch.float64, device=X.device)
-    sig = tm._log_sigma()
+    sig = tm._sigmas(tm.skip_dimensions, log=True)
     for k in range(tm.D):
         tm._set_coeffs(k, tm.coeffs_nonmon[k], tm.coeffs_mon[k])
     ptr = lambda t: B.c_void_p(t.data_ptr())

@@ -1431,52 +1431,35 @@ class transport_map():
                 sl['event'].synchronize()
         return out_host.numpy()
 
-    # ================================================================== densities (separable only)
-    def _log_det_accumulate(self, acc, Xraw_t, n, Zt, mode, std_offset):
-        dS = self._empty(n)
-        for k in range(self.D):
-            self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
-            # NB the reference evaluates the derivative basis on the UNstandardised samples (tm.py:2627, 2695)
-            B.check(self._lib.ttm_sep_eval(self._plans[k], None, 0, n, None, B.c_void_p(Xraw_t.data_ptr()),
-                                           Xraw_t.shape[1], B.c_void_p(dS.data_ptr()), self._stream()))
-            sigma = float(self.X_std[k + std_offset]) if self.standardize_samples else None
-            if sigma is None:
-                sigma = float(self.X_std[k + std_offset])        # AttributeError like the reference
-            B.check(self._lib.ttm_density_accumulate(self._ctx, B.c_void_p(acc.data_ptr()),
-                                                     B.c_void_p(Zt[k].data_ptr()) if Zt is not None else None,
-                                                     B.c_void_p(dS.data_ptr()), sigma, mode, n, self._stream()))
-
-    def evaluate_pullback_density(self, X, X_star=None):
-        """tm.py:2646-2712."""
-        assert self.monotonicity == "separable monotonicity", "evaluate_pushforward_density is currently only implemented for monotonicity = 'separable monotonicity'."
-        X = self._samples(X, ncol=self._Dtot if X_star is None else None)
-        dev = isinstance(X, _DevSamples)
-        X = self._stack(X_star, X)
-        if dev and X.n == 0:
-            return self._empty(0)
-        if self._fused_small():
-            return self._map_fused(X, 0, sigma=[float(self.X_std[k]) for k in range(self.D)])[1]   # X_std[k], tm.py:2706
-        n = X.shape[0]
-        torch = self._torch
-        if self.standardize_samples:
-            Xt = self._to_colmajor(X, self._mean_d, self._std_d)
+    # ================================================================== densities
+    def _density_input(self, X, X_star, ncol, msg='X has shape %s; the map expects %d columns'):
+        """A density evaluator's sample argument as a host float64 array or a _DevSamples, with its n and whether the
+        result stays on the device.  X and X_star are checked before any launch (ValueError; `msg` for X's columns): X
+        is 2-D with `ncol` columns and X_star holds the conditioning columns of a partial map, (n, skip_dimensions).
+        ncol=None is the reference's pullback, whose np.column_stack (tm.py:2675) takes any split of a row and a 1-D
+        host operand as one column: X and X_star then have n rows and together the map's skip_dimensions + D columns."""
+        X = self._samples(X, ncol=ncol)
+        shape = tuple(X.shape)
+        star = None if X_star is None else (tuple(X_star.shape) if hasattr(X_star, 'shape') else np.shape(X_star))
+        if ncol is None:
+            dims = (2,) if isinstance(X, _DevSamples) else (1, 2)
+            width = lambda s: s[1] if len(s) == 2 else 1
+            if (len(shape) not in dims or len(star) not in dims or star[0] != shape[0]
+                    or width(star) + width(shape) != self._Dtot):
+                raise ValueError('operands could not be broadcast together: X_star %s and X %s, the map has %d columns'
+                                 % (star, shape, self._Dtot))
         else:
-            Xt, n = self._Xt, self._N
-        Xraw_t = self._to_colmajor(X)
-        Zt = self._empty(self.D, n)
-        for k in range(self.D):
-            self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
-            self._s_device(k, Xt, n, Zt[k])
-        acc = torch.zeros(n, dtype=torch.float64, device=self._device)
-        self._log_det_accumulate(acc, Xraw_t, n, Zt, 0, 0)      # X_std[k] (not k+skip), tm.py:2706
-        out = self._empty(n)
-        B.check(self._lib.ttm_density_finish(self._ctx, B.c_void_p(acc.data_ptr()), None,
-                                             B.c_void_p(out.data_ptr()), n, self._stream()))
-        return self._result(out, dev)
+            if len(shape) != 2 or shape[1] != ncol:
+                raise ValueError(msg % (shape, ncol))
+            skip = self.skip_dimensions
+            if star is not None and (skip == 0 or star != (shape[0], skip)):
+                raise ValueError('X_star must have shape (%d, skip_dimensions = %d), got %s' % (shape[0], skip, star))
+        return X, shape[0], isinstance(X, _DevSamples)
 
-    def _stack(self, X_star, X):
-        """[X_star | X] (np.column_stack of tm.py:2614 / :2675) in the kind of X (host array or _DevSamples); with a
-        CUDA X the column count is checked before the device copy."""
+    def _stacked(self, X_star, X):
+        """[X_star | X] (np.column_stack of tm.py:2614 / :2675) in the kind of X: a host array, or a _DevSamples for a
+        CUDA tensor, whose device copy must hold the map's skip_dimensions + D columns."""
+        X = self._samples(X)
         if X_star is None:
             return X
         torch = self._torch
@@ -1491,75 +1474,95 @@ class transport_map():
         xs = Xs.t if isinstance(Xs, _DevSamples) else self._upload(Xs)
         return self._samples(torch.cat((xs.to(torch.float64), X.t.to(torch.float64)), dim=1))
 
-    def evaluate_pushforward_density(self, Z, log_target_pdf, X_star=None):
-        """tm.py:2569-2644.  `log_target_pdf` is a user Python callback, called with the inverse-mapped samples: a
-        host array, or a CUDA tensor when Z is one (it may then return a CUDA tensor or a host array of length n)."""
-        assert self.monotonicity == "separable monotonicity", "evaluate_pushforward_density is currently only implemented for monotonicity = 'separable monotonicity'."
-        torch = self._torch
-        dev = isinstance(Z, torch.Tensor) and Z.is_cuda
-        X = self.inverse_map(Z, X_star)
-        n = X.shape[0]
-        if dev and n == 0:
-            return self._empty(0)
-        log_target = log_target_pdf(X)
-        if isinstance(log_target, torch.Tensor) and log_target.is_cuda:
-            lt = log_target.to(self._device, torch.float64).reshape(-1).contiguous()
-        else:
-            lt = self._upload(np.ascontiguousarray(log_target, dtype=np.float64))
-        if dev and lt.numel() != n:
-            raise ValueError('log_target_pdf returned %d values for %d samples' % (lt.numel(), n))
-        X = self._stack(X_star, self._samples(X) if dev else X)
-        if self._fused_small():
-            return self._map_fused(X, 1, sigma=[float(self.X_std[k + self.skip_dimensions]) for k in range(self.D)],
-                                   log_target=lt)[1]                                  # X_std[k+skip], tm.py:2638
-        Xraw_t = self._to_colmajor(X)
-        acc = torch.zeros(n, dtype=torch.float64, device=self._device)
-        self._log_det_accumulate(acc, Xraw_t, n, None, 1, self.skip_dimensions)   # X_std[k+skip], tm.py:2638
-        out = self._empty(n)
-        B.check(self._lib.ttm_density_finish(self._ctx, B.c_void_p(acc.data_ptr()), B.c_void_p(lt.data_ptr()),
-                                             B.c_void_p(out.data_ptr()), n, self._stream()))
-        return self._result(out, dev)
-
-    # ================================================================== log densities (both monotonicity modes)
-    def _log_sigma(self):
-        """sigma_c = X_std[skip + k] per component (1 without standardisation)."""
-        if not self.standardize_samples:
+    def _sigmas(self, offset, log=False):
+        """sigma_k = X_std[offset + k] of every component; 1 for the log densities of a map without standardisation.
+        The reference's evaluators read X_std regardless (AttributeError on a map that never standardised)."""
+        if log and not self.standardize_samples:
             return [1.0] * self.D
-        return [float(self.X_std[k + self.skip_dimensions]) for k in range(self.D)]
+        return [float(self.X_std[k + offset]) for k in range(self.D)]
 
-    def _check_x_star(self, X_star, n):
-        """X_star of the log-density evaluators: the conditioning columns of a partial map, (n, skip_dimensions)."""
-        skip = self.skip_dimensions
-        if X_star is None:
-            return
-        shape = tuple(X_star.shape) if hasattr(X_star, 'shape') else np.shape(X_star)
-        if skip == 0 or len(shape) != 2 or shape[1] != skip or shape[0] != n:
-            raise ValueError('X_star must have shape (%d, skip_dimensions = %d), got %s' % (n, skip, shape))
+    def _log_target(self, log_target_pdf, X, n):
+        """log_target_pdf(X) as a float64 device vector; the callback returns n values as a host array or a CUDA
+        tensor (anything else would make the kernels read past the vector)."""
+        torch = self._torch
+        lt = log_target_pdf(X)
+        if isinstance(lt, torch.Tensor) and lt.is_cuda:
+            lt = lt.to(self._device, torch.float64).reshape(-1).contiguous()
+        else:
+            lt = self._upload(np.ascontiguousarray(lt, dtype=np.float64).reshape(-1))
+        if lt.numel() != n:
+            raise ValueError('log_target_pdf returned %d values for %d samples' % (lt.numel(), n))
+        return lt
 
-    def _log_det_terms(self, acc, Xt, n, mode):
-        """acc += sum_k [-S_k^2/2 - log(2 pi)/2 + l_k - log sigma_c] (mode 0) or acc -= sum_k [l_k - log sigma_c]
-        (mode 1) on the standardised column-major samples Xt, l_k = log d_c S_k."""
+    def _log_det(self, acc, Xs, Xd, n, mode, sigmas):
+        """The per-component log-determinant loop on n column-major samples: acc += sum_k [-S_k^2/2 - log(2 pi)/2 + l_k -
+        log sigma_k] (mode 0, S_k on the columns of Xs) or acc -= sum_k [l_k - log sigma_k] (mode 1), l_k = log dS_k/dx_c
+        on the columns of Xd: K-sep-eval and ttm_density_accumulate, or K-logdet-IR for integrated-rectifier maps."""
         ir = self.monotonicity == "integrated rectifier"
         S = self._empty(n) if mode == 0 else None
         dS = None if ir else self._empty(n)
         ptr = lambda t: B.c_void_p(t.data_ptr()) if t is not None else None
         st = self._stream()
-        for k, sigma in enumerate(self._log_sigma()):
+        for k, sigma in enumerate(sigmas):
             self._set_coeffs(k, self.coeffs_nonmon[k], self.coeffs_mon[k])
             if S is not None:
-                self._s_device(k, Xt, n, S)
+                self._s_device(k, Xs, n, S)
             if ir:
-                B.check(self._lib.ttm_ir_logdet_accumulate(self._plans[k], ptr(Xt), Xt.shape[1], n, ptr(S), sigma,
+                B.check(self._lib.ttm_ir_logdet_accumulate(self._plans[k], ptr(Xd), Xd.shape[1], n, ptr(S), sigma,
                                                            mode, ptr(acc), st))
             else:
-                B.check(self._lib.ttm_sep_eval(self._plans[k], None, 0, n, None, ptr(Xt), Xt.shape[1], ptr(dS), st))
+                B.check(self._lib.ttm_sep_eval(self._plans[k], None, 0, n, None, ptr(Xd), Xd.shape[1], ptr(dS), st))
                 B.check(self._lib.ttm_density_accumulate(self._ctx, ptr(acc), ptr(S), ptr(dS), sigma, mode, n, st))
 
-    def _standardized_colmajor(self, X):
-        if self.standardize_samples:
-            return self._to_colmajor(X, self._mean_d, self._std_d)
-        return self._to_colmajor(X)
+    def _density_finish(self, acc, lt, n, dev):
+        """exp(acc) (pullback) or exp(lt + acc) (pushforward) of the reference's evaluators."""
+        out = self._empty(n)
+        B.check(self._lib.ttm_density_finish(self._ctx, B.c_void_p(acc.data_ptr()),
+                                             B.c_void_p(lt.data_ptr()) if lt is not None else None,
+                                             B.c_void_p(out.data_ptr()), n, self._stream()))
+        return self._result(out, dev)
 
+    def evaluate_pullback_density(self, X, X_star=None):
+        """tm.py:2646-2712."""
+        assert self.monotonicity == "separable monotonicity", "evaluate_pushforward_density is currently only implemented for monotonicity = 'separable monotonicity'."
+        X, n, dev = self._density_input(X, X_star, self._Dtot if X_star is None else None)
+        if n == 0:
+            return self._empty(0) if dev else np.empty(0)
+        X = self._stacked(X_star, X)
+        if self._fused_small():
+            return self._map_fused(X, 0, sigma=self._sigmas(0))[1]                # X_std[k] (not k+skip), tm.py:2706
+        if self.standardize_samples:
+            Xs = self._to_colmajor(X, self._mean_d, self._std_d)
+        else:
+            Xs, n = self._Xt, self._N        # S on the stored ensemble, as the reference's map() (tm.py:2419-2422)
+        Xd = self._to_colmajor(X)            # NB the reference differentiates on the UNstandardised samples (tm.py:2695)
+        acc = self._torch.zeros(n, dtype=self._torch.float64, device=self._device)
+        self._log_det(acc, Xs, Xd, n, 0, self._sigmas(0))
+        return self._density_finish(acc, None, n, dev)
+
+    def evaluate_pushforward_density(self, Z, log_target_pdf, X_star=None):
+        """tm.py:2569-2644.  `log_target_pdf` is a user Python callback, called with the inverse-mapped samples: a
+        host array, or a CUDA tensor when Z is one (it may then return a CUDA tensor or a host array of length n)."""
+        assert self.monotonicity == "separable monotonicity", "evaluate_pushforward_density is currently only implemented for monotonicity = 'separable monotonicity'."
+        Z = self._samples(Z)
+        dev = isinstance(Z, _DevSamples)
+        if not dev and Z.shape[0] == 0:
+            return np.empty(0)
+        X = self.inverse_map(Z, X_star)          # its checks decide which Z and X_star go together, as tm.py:2614
+        n = X.shape[0]
+        if n == 0:
+            return self._empty(0)
+        lt = self._log_target(log_target_pdf, X, n)
+        X = self._stacked(X_star, X)
+        sigmas = self._sigmas(self.skip_dimensions)                                # X_std[k+skip], tm.py:2638
+        if self._fused_small():
+            return self._map_fused(X, 1, sigma=sigmas, log_target=lt)[1]
+        Xd = self._to_colmajor(X)                                                # unstandardised, tm.py:2627
+        acc = self._torch.zeros(n, dtype=self._torch.float64, device=self._device)
+        self._log_det(acc, None, Xd, n, 1, sigmas)
+        return self._density_finish(acc, lt, n, dev)
+
+    # ================================================================== log densities (both monotonicity modes)
     def evaluate_log_pullback_density(self, X, X_star=None):
         """log rho(x) = sum_k [-S_k(x~)^2/2 - log(2 pi)/2 + l_k(x~) - log sigma_c], the log density the fitted map pulls
         back from the standard Gaussian, for both monotonicity modes (DESIGN.md section 1).
@@ -1573,21 +1576,16 @@ class transport_map():
         X_star; X then has D columns, otherwise skip_dimensions + D.  X / X_star: host arrays or CUDA tensors; the
         result (n,) float64 follows X.  Unlike evaluate_pullback_density it returns the log (no underflow in high
         dimension) and differentiates the map it evaluates."""
-        X = self._samples(X, ncol=self._Dtot if X_star is None else self.D)
-        dev = isinstance(X, _DevSamples)
-        if X.ndim != 2 or X.shape[1] != (self._Dtot if X_star is None else self.D):
-            raise ValueError('X has shape %s; the map expects %d columns' %
-                             (tuple(X.shape), self._Dtot if X_star is None else self.D))
-        n = X.shape[0]
-        self._check_x_star(X_star, n)
+        X, n, dev = self._density_input(X, X_star, self._Dtot if X_star is None else self.D)
         if n == 0:
             return self._empty(0) if dev else np.empty(0)
-        X = self._stack(X_star, X)
+        X = self._stacked(X_star, X)
+        sigmas = self._sigmas(self.skip_dimensions, log=True)
         if self._fused_small():
-            return self._map_fused(X, 3, sigma=self._log_sigma())[1]
-        Xt = self._standardized_colmajor(X)
+            return self._map_fused(X, 3, sigma=sigmas)[1]
+        Xt = self._to_colmajor(X, self._mean_d, self._std_d) if self.standardize_samples else self._to_colmajor(X)
         acc = self._torch.zeros(n, dtype=self._torch.float64, device=self._device)
-        self._log_det_terms(acc, Xt, n, 0)
+        self._log_det(acc, Xt, Xt, n, 0, sigmas)
         return self._result(acc, dev)
 
     def evaluate_log_pushforward_density(self, Z, log_target_pdf, X_star=None):
@@ -1596,29 +1594,18 @@ class transport_map():
         as in evaluate_log_pullback_density).  `log_target_pdf` is called with the inverse-mapped samples (n, D) in the
         caller's units: a host array, or a CUDA tensor when Z is one; it returns n values (host array or CUDA
         tensor).  The result (n,) float64 follows Z."""
-        torch = self._torch
-        Z = self._samples(Z, ncol=self.D)
-        dev = isinstance(Z, _DevSamples)
-        if Z.ndim != 2 or Z.shape[1] != self.D:
-            raise ValueError('Z has shape %s; the map has %d components' % (tuple(Z.shape), self.D))
-        n = Z.shape[0]
-        self._check_x_star(X_star, n)
+        Z, n, dev = self._density_input(Z, X_star, self.D, 'Z has shape %s; the map has %d components')
         if n == 0:
             return self._empty(0) if dev else np.empty(0)
         X = self.inverse_map(Z, X_star)
-        log_target = log_target_pdf(X)
-        if isinstance(log_target, torch.Tensor) and log_target.is_cuda:
-            lt = log_target.to(self._device, torch.float64).reshape(-1).contiguous()
-        else:
-            lt = self._upload(np.ascontiguousarray(log_target, dtype=np.float64).reshape(-1))
-        if lt.numel() != n:
-            raise ValueError('log_target_pdf returned %d values for %d samples' % (lt.numel(), n))
-        X = self._stack(X_star, self._samples(X) if dev else X)
+        lt = self._log_target(log_target_pdf, X, n)
+        X = self._stacked(X_star, X)
+        sigmas = self._sigmas(self.skip_dimensions, log=True)
         if self._fused_small():
-            return self._map_fused(X, 4, sigma=self._log_sigma(), log_target=lt)[1]
-        Xt = self._standardized_colmajor(X)
+            return self._map_fused(X, 4, sigma=sigmas, log_target=lt)[1]
+        Xt = self._to_colmajor(X, self._mean_d, self._std_d) if self.standardize_samples else self._to_colmajor(X)
         acc = lt.clone()
-        self._log_det_terms(acc, Xt, n, 1)
+        self._log_det(acc, None, Xt, n, 1, sigmas)
         return self._result(acc, dev)
 
     # ================================================================== measurement helpers
